@@ -3,6 +3,7 @@
 scans at 0.05 m voxels (BASELINE.json's metric), one scan per step.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our engine (one JSON line)
+  python bench.py ... --dump-outputs DIR                       ... and the resulting map as DIR/*.npy
   python bench.py --impl reference ...                         the reference's own CPU
                                                                MergedTsdfIntegrator (oracle/_ref)
 Multi-GPU runs are launched by torchrun, one rank per GPU (DESIGN.md "multi-GPU").
@@ -358,6 +359,38 @@ def measure_traffic(conf_name, timeout_s=300, cache_control="all"):
                  "  (caches left as the previous kernel left them, as in the real run)") + ", run inside this bench"}
 
 
+# ------------------------------------------------------------------ output dump
+DUMP_MAX_BLOCKS = 384   # sampled blocks: 4096 voxels x (4 + 4 + 16 B TSDF + 8 B ESDF) each, ~48 MB in all
+
+
+def dump_outputs(out_dir, layer, esdf_layer=None):
+    """The map a caller of the timed path holds after its last step, as .npy files: every allocated block index
+    and, for a seeded sample of at most DUMP_MAX_BLOCKS of those blocks (all of them when there are fewer), the
+    voxels.  Block indices are sorted, so two builds with the same map dump the same sample."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a, dtype):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=dtype))
+
+    for prefix, lay in (("tsdf", layer), ("esdf", esdf_layer)):
+        if lay is None:
+            continue
+        idx = lay.getAllAllocatedBlocks()
+        pick = np.arange(len(idx))
+        if len(idx) > DUMP_MAX_BLOCKS:
+            pick = np.sort(np.random.default_rng(0).choice(len(idx), DUMP_MAX_BLOCKS, replace=False))
+        vox, upd = lay.getBlocks(idx[pick])
+        save(prefix + "_block_indices", idx, np.float64)
+        save(prefix + "_sample_block_indices", idx[pick], np.float64)
+        save(prefix + "_sample_updated", upd, np.float32)
+        save(prefix + "_sample_distance", vox["distance"], np.float32)
+        if prefix == "tsdf":
+            save("tsdf_sample_weight", vox["weight"], np.float32)
+            save("tsdf_sample_color", vox["color"], np.float32)
+        else:
+            save("esdf_sample_observed", vox["observed"], np.float32)
+
+
 # --------------------------------------------------------------------------- ours
 STAGE_OF_KERNEL = {  # stage name (Layer.stageMs) -> kernels that run in it
     "point_keys": ("k_point_bounds", "k_point_keys"), "point_sort": ("k_sort",),
@@ -451,6 +484,8 @@ def run_ours(args, conf, rank, world):
         K += c["updates"]
     sync_ms = layer.timerStopMs()
     barrier()
+    if do_esdf and args.dump_outputs and rank == 0:  # with the ESDF update after every scan this is the timed path
+        dump_outputs(args.dump_outputs, layer, esdf_layer)
     del layer, integ, esdf_int
     # ---- (1b) headline: the same K scans submitted back to back (vbx_tsdf_integrate_async): stages of
     # neighbouring scans overlap; timed on the device until the last scan is in the map.  With the ESDF
@@ -482,6 +517,8 @@ def run_ours(args, conf, rank, world):
         last_counters = integ.counters()
         launches = last_counters["kernel_launches_total"] - launches_before
         n_blocks = layer.getNumberOfAllocatedBlocks()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, layer)
     clocks = sampler.stop() if rank == 0 else None
     dev_ms, wall_ms, sync_ms = reduce_max(dev_ms, wall_ms, sync_ms)
     value = pts_timed / (dev_ms * 1e-3)
@@ -752,7 +789,11 @@ def main():
     ap.add_argument("--trunc", type=float, default=None, help="override default_truncation_distance (C2: 4.0 = the literal '4 m')")
     ap.add_argument("--no-traffic", dest="traffic", action="store_false", help="skip the ncu DRAM-traffic pass")
     ap.add_argument("--traffic-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the map they produced as DIR/<name>.npy (with N > 1: rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     conf = dict(CONFIGS[args.config])
     if args.trunc is not None:

@@ -1,9 +1,37 @@
 """Comparison helpers shared by the parity tests, smoke() and bench.py."""
 from __future__ import annotations
 
+import hashlib
 from typing import Dict
 
 import numpy as np
+
+
+def layer_digest(indices: np.ndarray, voxels: np.ndarray, updated: np.ndarray = None) -> str:
+    """SHA-256 of a layer: its sorted block indices, the voxel bytes of those blocks in that order and, when
+    given, their updated bits.  Equal digests mean bit-identical layers."""
+    h = hashlib.sha256()
+    h.update(np.ascontiguousarray(indices, dtype=np.int32).tobytes())
+    h.update(np.ascontiguousarray(voxels).tobytes())
+    if updated is not None:
+        h.update(np.ascontiguousarray(updated, dtype=np.uint8).tobytes())
+    return h.hexdigest()
+
+
+def device_layer_digest(layer, with_updated: bool = False) -> str:
+    """layer_digest of a GPU Layer (voxblox_b200.Layer)."""
+    idx = layer.getAllAllocatedBlocks()
+    vox, upd = layer.getBlocks(idx)
+    return layer_digest(idx, vox, upd if with_updated else None)
+
+
+def oracle_layer_digest(omap, layer: int = 0, with_updated: bool = False) -> str:
+    """layer_digest of an oracle map's TSDF (0) or ESDF (1) layer."""
+    idx = omap.block_indices(layer)
+    blocks = [omap.block(i, layer) for i in idx]
+    vox = np.stack([b[0] for b in blocks]) if blocks else np.zeros(0)
+    upd = np.array([b[1] for b in blocks], dtype=np.uint8)
+    return layer_digest(idx, vox, upd if with_updated else None)
 
 
 def rel_err(a: np.ndarray, b: np.ndarray, floor: float) -> np.ndarray:

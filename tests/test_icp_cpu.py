@@ -12,6 +12,7 @@ import pytest
 from oracle import pyoracle as po
 from tests.golden import make_golden as mg
 from tests.golden import make_icp_golden as mi
+from tests.golden import make_reference_golden as mr
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = json.load(open(os.path.join(HERE, "golden", "icp.json")))
@@ -39,14 +40,15 @@ def test_port_icp_matches_reference_library(name):
     assert np.abs(rq - pq).max() <= TOL and np.abs(rt - pt).max() <= TOL
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built")
 def test_shuffle_is_the_library_shuffle():
-    """both checkers call std::shuffle(std::default_random_engine(seed)) of the C++ library they are built with"""
-    for n, seed in ((0, 1), (1, 1), (1000, 42), (4099, 7)):
-        a, b = np.zeros(n, np.uint32), np.zeros(n, np.uint32)
-        po.OracleLib("reference").lib.vbo_icp_shuffle(n, seed, a.ctypes.data)
-        po.OracleLib("port").lib.vbo_icp_shuffle(n, seed, b.ctypes.data)
-        assert (a == b).all() and sorted(a.tolist()) == list(range(n))
+    """both checkers call std::shuffle(std::default_random_engine(seed)) of the C++ library they are built with;
+    the reference's permutations are stored as a digest by tests/golden/make_reference_golden.py"""
+    port = po.OracleLib("port")
+    for n, seed in mr.SHUFFLES:
+        b = np.zeros(n, np.uint32)
+        port.lib.vbo_icp_shuffle(n, seed, b.ctypes.data)
+        assert sorted(b.tolist()) == list(range(n))
+    assert mr.shuffle_digest(port) == mr.golden("restatement_pins", "shuffle")
 
 
 def test_round_robin_schedule_with_one_thread_is_the_sequential_algorithm():

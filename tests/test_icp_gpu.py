@@ -7,15 +7,16 @@ dependent fusions: the bound is the north-star float tolerance, 1e-4 -- absolute
 coefficients, relative to max(1, |t|) on the translation -- not bit identity.  The TSDF maps the two sides
 match against ARE bit identical (Merged, asserted).
 
-num_threads = 1 is the reference's only deterministic setting and is compared with the reference itself;
-num_threads = T > 1 is compared with the restatement's round-robin schedule (oracle/vbo_api.h), which the
+num_threads = 1 is the reference's only deterministic setting and is compared with the reference itself (its
+map digest and refined poses, stored by tests/golden/make_reference_golden.py); num_threads = T > 1 is compared with the restatement's round-robin schedule (oracle/vbo_api.h), which the
 device implements with T warps."""
 import numpy as np
 import pytest
 
 import voxblox_b200 as vb
 from oracle import pyoracle as po
-from tests.parity import compare_tsdf
+from tests.golden import make_reference_golden as mr
+from tests.parity import compare_tsdf, device_layer_digest
 from voxblox_b200 import scenes
 
 pytestmark = pytest.mark.gpu
@@ -23,13 +24,19 @@ pytestmark = pytest.mark.gpu
 TOL = 1e-4
 
 
-def _maps(which, voxel, trunc, scans):
+def _device_map(voxel, trunc, scans):
     cfg = vb.TsdfIntegratorConfig(default_truncation_distance=trunc, integrator_threads=1)
     layer = vb.Layer(voxel, 16)
     integ = vb.TsdfIntegratorFactory.create("merged", cfg, layer)
-    omap = po.OracleMap(po.OracleLib(which), po.TsdfConfig(default_truncation_distance=trunc, integrator_threads=1), voxel, 16)
     for s in scans:
         integ.integratePointCloud((s[2], s[3]), s[0], s[1])
+    return layer
+
+
+def _maps(which, voxel, trunc, scans):
+    layer = _device_map(voxel, trunc, scans)
+    omap = po.OracleMap(po.OracleLib(which), po.TsdfConfig(default_truncation_distance=trunc, integrator_threads=1), voxel, 16)
+    for s in scans:
         omap.integrate(po.MERGED, s)
     rep = compare_tsdf(layer, omap)
     assert rep["blocks_equal"] and rep["n_bit_exact"] == rep["n_voxels"], rep
@@ -51,18 +58,25 @@ def _perturbed(s, dt, yaw):
     return w.astype(np.float32), (np.asarray(s[3], np.float64) + np.asarray(dt)).astype(np.float32)
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built (no /root/reference here)")
+# (translation, yaw) added to the fourth scan's true pose before refinement
+PERTURBATIONS = [((0, 0, 0), 0.0), ((0.03, -0.02, 0.01), 0.0), ((-0.02, 0.03, 0.0), 0.01)]
+
+
 @pytest.mark.parametrize("refine_roll_pitch", [0, 1])
 def test_icp_one_thread_against_the_reference(refine_roll_pitch):
     """640 x 480 room scans at 0.05 m (the bench workload): map of three scans, the fourth cloud refined from
     its true pose and from two perturbed ones."""
     ss = [scenes.c3_room_scan(i) for i in range(4)]
-    layer, omap = _maps("reference", 0.05, 0.2, ss[:3])
+    gold = mr.golden("icp", f"refine_roll_pitch_{refine_roll_pitch}")
+    mr.require_inputs(ss, gold)
+    layer = _device_map(0.05, 0.2, ss[:3])
+    assert device_layer_digest(layer) == gold["map"]   # bit-identical to the reference's map
     s = ss[3]
-    for k, (dt, yaw) in enumerate([((0, 0, 0), 0.0), ((0.03, -0.02, 0.01), 0.0), ((-0.02, 0.03, 0.0), 0.01)]):
+    for k, ((dt, yaw), g) in enumerate(zip(PERTURBATIONS, gold["runs"])):
         q0, t0 = _perturbed(s, dt, yaw)
         dev = vb.ICP(vb.ICPConfig(refine_roll_pitch=refine_roll_pitch)).runICP(layer, s[0], (q0, t0), seed=7 + k)
-        ref = omap.icp(po.IcpConfig(refine_roll_pitch=refine_roll_pitch), s[0], q0, t0, 7 + k)
+        ref = (np.array([float.fromhex(v) for v in g["q_wxyz"]], np.float32),
+               np.array([float.fromhex(v) for v in g["t"]], np.float32), g["num_updates"])
         rep = _close(dev, ref)
         err0 = float(np.abs(t0 - s[3]).max())
         err1 = float(np.abs(dev[1][1] - s[3]).max())

@@ -1,7 +1,7 @@
 """Pins the meshing restatement (oracle/vbx_oracle.cc, generateMesh) and the generated marching-cubes
 table (voxblox_b200/csrc/vbx_mc_tables.h) to the reference: MeshIntegrator<TsdfVoxel>
 (mesh/mesh_integrator.h), MarchingCubes (mesh/marching_cubes.h, src/mesh/marching_cubes.cc) compiled
-from /root/reference into oracle/_ref, and committed digests where the reference is absent."""
+from the reference's sources into oracle/_ref, and committed digests where the reference is absent."""
 import ctypes as C
 import hashlib
 import json
@@ -46,15 +46,13 @@ def test_generated_table_is_well_formed():
         assert sorted(set(v for v in rows[case] if v >= 0)) == sorted(set(v for v in rows[255 - case] if v >= 0))
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built (no /root/reference here)")
 def test_generated_table_equals_reference_table():
-    lib = po.OracleLib("reference").lib
-    tri = np.zeros(256 * 16, dtype=np.int32)
-    edges = np.zeros(24, dtype=np.int32)
-    assert lib.vbo_mc_tables(tri.ctypes.data, edges.ctypes.data) == 0
+    """The packed tables against a digest of the reference's MarchingCubes::kTriangleTable / kEdgeIndexPairs
+    (stored by tests/golden/make_reference_golden.py)."""
+    from tests.golden import make_reference_golden as mr
+
     rows, pairs = _packed_tables()
-    assert tri.reshape(256, 16).tolist() == rows
-    assert [tuple(p) for p in edges.reshape(12, 2).tolist()] == pairs
+    assert mr.int32_digest(rows, pairs) == mr.golden("restatement_pins", "mc_tables")
 
 
 def _meshed_map(which, use_color=True, incremental=True):

@@ -2,8 +2,8 @@
 trusts -- against the reference itself:
   * bit-identical layers vs oracle/_ref (the reference's own integrator sources compiled
     against oracle/shim/), wherever that library exists (it travels to the GPU box);
-  * the committed digests of tests/golden/digests.json, generated from oracle/_ref by
-    tests/golden/make_golden.py, everywhere;
+  * the committed digests of tests/golden/digests.json and tests/golden/reference.json, generated
+    from oracle/_ref by tests/golden/make_golden.py and make_reference_golden.py, everywhere;
   * the known-answer INDEXING vectors of the reference's test/test_tsdf_map.cc.
 """
 import json
@@ -14,6 +14,8 @@ import pytest
 
 from oracle import pyoracle as po
 from tests.golden import make_golden as mg
+from tests.golden import make_reference_golden as mr
+from tests.parity import oracle_layer_digest
 from voxblox_b200 import scenes
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -39,91 +41,91 @@ def test_port_matches_reference_library(name):
     assert ref == port, name
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built")
-def test_port_matches_reference_voxelwise_with_esdf():
-    """Same comparison voxel by voxel (readable failure) incl. updated bits, over more scans."""
+def voxelwise_with_esdf_maps(lib):
+    """Simple / Merged / Fast, each followed by an incremental ESDF update, over four scans."""
     scans = scenes.c3_room_sequence(n_scans=4, width=128, height=96)
     cfg = po.TsdfConfig(default_truncation_distance=0.4, integrator_threads=1)
     ecfg = po.EsdfConfig(max_distance_m=4.0, default_distance_m=4.0, min_distance_m=0.2, min_diff_m=0.0, multi_queue=1)
+    maps = {}
     for kind in (1, 2, 3):
-        a = po.OracleMap(po.OracleLib("reference"), cfg, 0.1, 16)
-        b = po.OracleMap(po.OracleLib("port"), cfg, 0.1, 16)
-        a.esdf_create(ecfg)
-        b.esdf_create(ecfg)
+        m = maps[kind] = po.OracleMap(lib, cfg, 0.1, 16)
+        m.esdf_create(ecfg)
         for s in scans:
-            a.integrate(kind, s)
-            b.integrate(kind, s)
-            a.esdf_update(False, True)
-            b.esdf_update(False, True)
-        for layer in (0, 1):
-            ia, ib = a.block_indices(layer), b.block_indices(layer)
-            assert ia.shape == ib.shape and (ia == ib).all()
-            for i in ia:
-                va, ua = a.block(i, layer)
-                vb, ub = b.block(i, layer)
-                assert ua == ub
-                assert va.tobytes() == vb.tobytes(), (kind, layer, tuple(i))
+            m.integrate(kind, s)
+            m.esdf_update(False, True)
+    return maps
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built")
-def test_port_matches_reference_esdf_blocks_and_setters():
-    """updateFromTsdfBlocks on a block subset, setEsdfMaxDistance / setFullEuclidean, then batch."""
+def esdf_blocks_and_setters_maps(lib):
+    """updateFromTsdfBlocks on a block subset (map 1 of 2), then setEsdfMaxDistance / setFullEuclidean and a
+    batch update (map 2 of 2)."""
     scans = scenes.c3_room_sequence(n_scans=3, width=96, height=72)
     cfg = po.TsdfConfig(default_truncation_distance=0.4, integrator_threads=1)
     ecfg = po.EsdfConfig(max_distance_m=2.0, default_distance_m=2.0, min_distance_m=0.2, min_diff_m=1e-3)
-    maps = [po.OracleMap(po.OracleLib(w), cfg, 0.1, 16) for w in ("reference", "port")]
-    for m in maps:
+    maps = [po.OracleMap(lib, cfg, 0.1, 16) for _ in range(2)]
+    for k, m in enumerate(maps):
         m.esdf_create(ecfg)
         for s in scans:
             m.integrate(2, s)
         blocks = m.block_indices(0)
         m.esdf_update_blocks(np.concatenate([blocks[::2], np.array([[77, 77, 77]], np.int32)]), incremental=False)
-    a, b = maps
-    ia, ib = a.block_indices(1), b.block_indices(1)
-    assert ia.shape == ib.shape and (ia == ib).all()
-    assert all(a.block(i, 1)[0].tobytes() == b.block(i, 1)[0].tobytes() for i in ia)
-    for m in maps:
-        m.esdf_set_max_distance(3.0)
-        m.esdf_set_full_euclidean(True)
-        m.esdf_update(True, True)
-    ia, ib = a.block_indices(1), b.block_indices(1)
-    assert ia.shape == ib.shape and (ia == ib).all()
-    assert all(a.block(i, 1)[0].tobytes() == b.block(i, 1)[0].tobytes() for i in ia)
+        if k == 1:
+            m.esdf_set_max_distance(3.0)
+            m.esdf_set_full_euclidean(True)
+            m.esdf_update(True, True)
+    return maps
 
 
-@pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built")
+def serialization_map(lib):
+    scans = scenes.c3_room_sequence(n_scans=2, width=96, height=72)
+    m = po.OracleMap(lib, po.TsdfConfig(default_truncation_distance=0.4, integrator_threads=1), 0.1, 16)
+    m.esdf_create(po.EsdfConfig(max_distance_m=2.0, default_distance_m=2.0, min_distance_m=0.2))
+    for s in scans:
+        m.integrate(2, s)
+    m.esdf_update(False, True)
+    return m
+
+
+def serialization_decoded(lib, words, indices):
+    """A fresh map into which the serialized blocks of both layers were deserialized."""
+    m = po.OracleMap(lib, po.TsdfConfig(default_truncation_distance=0.4, integrator_threads=1), 0.1, 16)
+    m.esdf_create(po.EsdfConfig(max_distance_m=2.0, default_distance_m=2.0, min_distance_m=0.2))
+    for layer in (0, 1):
+        for i, w in zip(indices[layer], words[layer]):
+            m.deserialize_block(i, w, layer)
+    return m
+
+
+def test_port_matches_reference_voxelwise_with_esdf():
+    """Same comparison as the committed digests, incl. updated bits and an incremental ESDF, over more scans."""
+    gold = mr.restatement_golden()["voxelwise_with_esdf"]
+    for kind, m in voxelwise_with_esdf_maps(po.OracleLib("port")).items():
+        for layer in (0, 1):
+            assert oracle_layer_digest(m, layer, with_updated=True) == gold[str(kind)][layer], (kind, layer)
+
+
+def test_port_matches_reference_esdf_blocks_and_setters():
+    """updateFromTsdfBlocks on a block subset, setEsdfMaxDistance / setFullEuclidean, then batch."""
+    gold = mr.restatement_golden()["esdf_blocks_and_setters"]
+    for k, m in enumerate(esdf_blocks_and_setters_maps(po.OracleLib("port"))):
+        assert oracle_layer_digest(m, 1) == gold[k], k
+
+
 def test_port_matches_reference_block_serialization():
     """Block::serializeToIntegers / deserializeFromIntegers (src/core/block.cc) for both voxel types,
     incl. the sign-extension quirk of serializeDirection for negative parent components."""
-    scans = scenes.c3_room_sequence(n_scans=2, width=96, height=72)
-    cfg = po.TsdfConfig(default_truncation_distance=0.4, integrator_threads=1)
-    ecfg = po.EsdfConfig(max_distance_m=2.0, default_distance_m=2.0, min_distance_m=0.2)
-    ref, port = (po.OracleMap(po.OracleLib(w), cfg, 0.1, 16) for w in ("reference", "port"))
-    for m in (ref, port):
-        m.esdf_create(ecfg)
-        for s in scans:
-            m.integrate(2, s)
-        m.esdf_update(False, True)
-    saw_negative_parent = False
-    for layer in (0, 1):
-        for i in ref.block_indices(layer):
-            wr, wp = ref.serialize_block(i, layer), port.serialize_block(i, layer)
-            assert wr.tobytes() == wp.tobytes(), (layer, tuple(i))
-            if layer == 1:
-                saw_negative_parent |= bool((ref.block(i, 1)[0]["parent"] < 0).any())
-    assert saw_negative_parent
-    # round trip through fresh maps: reference and restatement decode the same words the same way
-    ref2, port2 = (po.OracleMap(po.OracleLib(w), cfg, 0.1, 16) for w in ("reference", "port"))
-    for m in (ref2, port2):
-        m.esdf_create(ecfg)
-    for layer in (0, 1):
-        for i in ref.block_indices(layer):
-            w = ref.serialize_block(i, layer)
-            ref2.deserialize_block(i, w, layer)
-            port2.deserialize_block(i, w, layer)
-            assert ref2.block(i, layer)[0].tobytes() == port2.block(i, layer)[0].tobytes()
-            if layer == 0:  # TSDF serialisation is lossless
-                assert ref2.block(i, 0)[0].tobytes() == ref.block(i, 0)[0].tobytes()
+    gold = mr.restatement_golden()["serialization"]
+    port = po.OracleLib("port")
+    m = serialization_map(port)
+    indices = [m.block_indices(layer) for layer in (0, 1)]
+    words = [[m.serialize_block(i, layer) for i in indices[layer]] for layer in (0, 1)]
+    assert [mr.int32_digest(*w) for w in words] == gold["words"]
+    assert any((m.block(i, 1)[0]["parent"] < 0).any() for i in indices[1])
+    # round trip through a fresh map: the restatement decodes the words as the reference does
+    decoded = serialization_decoded(port, words, indices)
+    assert [oracle_layer_digest(decoded, layer) for layer in (0, 1)] == gold["decoded"]
+    for i in indices[0]:  # TSDF serialisation is lossless
+        assert decoded.block(i, 0)[0].tobytes() == m.block(i, 0)[0].tobytes()
 
 
 def _integrate_single_point(point, voxel_size, vps):

@@ -8,20 +8,20 @@ standing on a ground plane, every integrator's layer compared with the analytic 
     reference's simulated camera; on the views used here the bound is max(1 %, what the reference's own
     integrators show on the same clouds), see the assertions),
   * min error ~ 0 (1e-4), max error < 2 truncation distances, rmse < 2 voxels.
-The same three integrators of the REFERENCE (oracle/_ref, one thread) run beside the device on the same
-clouds; Simple and Merged must be bit-identical to them (so their errors are equal by construction), and
-the Fast integrator -- statistical by design -- must meet the criteria with errors no worse than the
-reference's Fast.  The measured numbers are printed by every run."""
+The same three integrators of the REFERENCE (oracle/_ref, one thread) were run on the same clouds by
+tests/golden/make_reference_golden.py, which stores their layer digests and errors; Simple and Merged must
+be bit-identical to them (so their errors are equal by construction), and the Fast integrator --
+statistical by design -- must meet the criteria with errors no worse than the reference's Fast.  The
+measured numbers are printed by every run."""
 import numpy as np
 import pytest
 
 import voxblox_b200 as vb
-from oracle import pyoracle as po
-from tests.parity import compare_tsdf
+from tests.golden import make_reference_golden as mr
+from tests.parity import device_layer_digest
 from tests.test_esdf_reference_gpu import _gt_scans, _world_sdf
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not po.available("reference"), reason="oracle/_ref not built (no /root/reference here)")]
+pytestmark = pytest.mark.gpu
 
 KIND_ID = {"simple": 1, "merged": 2, "fast": 3}
 
@@ -50,21 +50,19 @@ def _evaluate(blocks, voxel, trunc):
 def test_tsdf_integrators_acceptance_criteria_vs_ground_truth(voxel):
     trunc = 4 * voxel                                        # test_sdf_integrators.cc:76
     scans = _gt_scans()
+    gold = mr.golden("tsdf_ground_truth", str(voxel))
+    mr.require_inputs(scans, gold)
     dev, ref = {}, {}
     for kind in ("simple", "merged", "fast"):
         cfg = vb.TsdfIntegratorConfig(default_truncation_distance=trunc, integrator_threads=1)
         layer = vb.Layer(voxel, 16)
         integ = vb.TsdfIntegratorFactory.create(kind, cfg, layer)
-        omap = po.OracleMap(po.OracleLib("reference"),
-                            po.TsdfConfig(default_truncation_distance=trunc, integrator_threads=1), voxel, 16)
         for s in scans:
             integ.integratePointCloud((s[2], s[3]), s[0], s[1])
-            omap.integrate(KIND_ID[kind], s)
         dev[kind] = _evaluate(layer.blocks(), voxel, trunc)
-        ref[kind] = _evaluate(omap.blocks(), voxel, trunc)
+        ref[kind] = gold[kind]["errors"]
         if kind != "fast":
-            rep = compare_tsdf(layer, omap)
-            assert rep["blocks_equal"] and rep["n_bit_exact"] == rep["n_voxels"] and rep["color_mismatch"] == 0, rep
+            assert device_layer_digest(layer) == gold[kind]["digest"], kind   # bit-identical to the reference
         print(f"voxel {voxel} {kind:7s} device {dev[kind]} | reference {ref[kind]}")
     total = dev["simple"]["overlapping"] + dev["simple"]["non_overlapping"]
     one_percent = int(total * 0.01)
