@@ -218,11 +218,18 @@ def _layer_bytes(layer):
 
 @pytest.mark.parametrize("kind", [1, 2])
 @pytest.mark.parametrize("pageable", [False, True])
-def test_async_submission_equals_synchronous(kind, pageable):
+@pytest.mark.parametrize("n_scans,rings", [(7, None), (23, None), (23, (2, 1))],
+                         ids=["7_scans", "23_scans", "23_scans_2_sets_1_lane"])
+def test_async_submission_equals_synchronous(kind, pageable, n_scans, rings, monkeypatch):
     """vbx_tsdf_integrate_async overlaps the front half of scan i+1 with the back half of scan i;
-    the map must equal the synchronous calls' bit for bit (and so the oracle's)."""
+    the map must equal the synchronous calls' bit for bit (and so the oracle's).  With more scans
+    than hand-off sets and front lanes every ring (sets, lanes, sort and copy streams) wraps at least
+    twice: a submission waits for the scan that used its set, collects it and reuses the buffers."""
+    if rings:
+        monkeypatch.setenv("VBX_ASYNC_SETS", str(rings[0]))
+        monkeypatch.setenv("VBX_ASYNC_LANES", str(rings[1]))
     cfg = vb.TsdfIntegratorConfig(default_truncation_distance=0.4, integrator_threads=1)
-    scans = scenes.c3_room_sequence(n_scans=7, width=160, height=120)
+    scans = scenes.c3_room_sequence(n_scans=n_scans, width=160, height=120)
     la, ls = vb.Layer(0.1, 16), vb.Layer(0.1, 16)
     ia = vb.TsdfIntegratorFactory.create(kind, cfg, la)
     isync = vb.TsdfIntegratorFactory.create(kind, cfg, ls)
@@ -278,7 +285,7 @@ def test_async_scan_with_more_updates_than_one_pass_is_redone_not_dropped(kind):
     ia, isync = vb.TsdfIntegratorFactory.create(kind, cfg, la), vb.TsdfIntegratorFactory.create(kind, cfg, ls)
     scans = scenes.c3_room_sequence(n_scans=9, width=96, height=72)
     keep = []
-    for s in scans:   # more scans than hand-off sets: the recovery also runs when a set is reused
+    for s in scans:   # fewer scans than the default ten hand-off sets: the recovery runs in la.sync()
         isync.integratePointCloud((s[2], s[3]), s[0], s[1])
         p, c = np.ascontiguousarray(s[0]), np.ascontiguousarray(s[1])
         keep.append((p, c))

@@ -65,7 +65,7 @@ static inline unsigned int grid_for(uint64_t n, int block) { return (unsigned in
 // The block hash rebuilt from slot_key: after removals, and after a call that ran out of pool slots
 // (its surplus hash entries have no slot and must not be found by later calls).
 int rebuild_hash(vbx_ctx* c) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   VBX_CUDA(c, cudaMemsetAsync(c->tab.hkeys, 0xff, (size_t)c->hcap * sizeof(uint64_t), s));
   VBX_CUDA(c, cudaMemsetAsync(c->tab.hslot, 0xff, (size_t)c->hcap * sizeof(int32_t), s));
   VBX_CUDA(c, cudaMemsetAsync(c->tab.htouch, 0, (size_t)c->hcap * sizeof(unsigned long long), s));
@@ -186,7 +186,7 @@ int upload_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m, const 
   if (m == 0) return VBX_OK;
   if (layer == VBX_LAYER_ESDF && !c->has_esdf) return fail(c, VBX_E_STATE, "no ESDF layer");
   if (m > c->tab.max_blocks) return fail(c, VBX_E_CAPACITY, "more blocks than the pool holds");
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   std::vector<uint64_t> keys(m);
   for (uint64_t i = 0; i < m; ++i) {
     const int32_t* p = idx3 + 3 * i;
@@ -196,20 +196,21 @@ int upload_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m, const 
     }
     keys[i] = pack3(p[0], p[1], p[2]);
   }
-  // scratch: the point-key buffer holds the keys, the ray list the hash positions, cnt the slots
+  // scratch of hand-off set 0: the point-key buffer holds the keys, the ray list the hash positions, cnt the slots
   if (m > c->max_points) return fail(c, VBX_E_CAPACITY, "upload more than max_points_per_scan blocks at once");
-  VBX_CUDA(c, cudaMemcpyAsync(c->pkeys[0], keys.data(), m * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-  VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
-  k_ensure_keys<<<grid_for(m, 256), 256, 0, s>>>(c->tab, c->pkeys[0], (uint32_t)m, c->ray_list, c->d_state);
+  vbx_ctx::ScratchSet& S = c->set[0];
+  VBX_CUDA(c, cudaMemcpyAsync(S.pkeys0, keys.data(), m * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  VBX_CUDA(c, cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), s));
+  k_ensure_keys<<<grid_for(m, 256), 256, 0, s>>>(c->tab, S.pkeys0, (uint32_t)m, S.ray_list, S.d_state);
   // a block inserted into the ESDF layer at an index the TSDF layer does not hold occupies a slot of its own
   k_assign_uploaded<<<grid_for(c->tab.max_blocks, 256), 256, 0, s>>>(
-      c->tab, c->n_blocks, layer == VBX_LAYER_ESDF ? kSlotNoTsdf : (uint8_t)0, c->d_state);
-  k_slots_of<<<grid_for(m, 256), 256, 0, s>>>(c->tab, c->ray_list, (uint32_t)m, reinterpret_cast<int32_t*>(c->cnt));
-  VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+      c->tab, c->n_blocks, layer == VBX_LAYER_ESDF ? kSlotNoTsdf : (uint8_t)0, S.d_state);
+  k_slots_of<<<grid_for(m, 256), 256, 0, s>>>(c->tab, S.ray_list, (uint32_t)m, reinterpret_cast<int32_t*>(S.cnt));
+  VBX_CUDA(c, cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
-  if (c->h_state->error & kFatalErrors) return fail(c, VBX_E_CAPACITY, "block pool / hash full during upload");
-  if (layer == VBX_LAYER_ESDF && c->h_state->n_new) c->maybe_esdf_only = true;
-  if (int rc = set_n_blocks(c, c->h_state->n_blocks)) return rc;
+  if (S.h_state->error & kFatalErrors) return fail(c, VBX_E_CAPACITY, "block pool / hash full during upload");
+  if (layer == VBX_LAYER_ESDF && S.h_state->n_new) c->maybe_esdf_only = true;
+  if (int rc = set_n_blocks(c, S.h_state->n_blocks)) return rc;
   const size_t bbytes = payload_bytes(c, layer, serialized);
   const uint32_t wpv = (layer == VBX_LAYER_TSDF) ? 3u : (serialized ? 1u : 5u);  // threads per voxel along x
   uint32_t* pool = layer == VBX_LAYER_TSDF ? reinterpret_cast<uint32_t*>(c->tab.tsdf) : reinterpret_cast<uint32_t*>(c->tab.esdf);
@@ -224,7 +225,7 @@ int upload_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m, const 
     if (updated_bits) VBX_CUDA(c, cudaMemcpyAsync(d_upd, updated_bits + at, k, cudaMemcpyHostToDevice, s));
     const dim3 grid(grid_for((uint64_t)wpv * c->vox_per_block, 256), (unsigned int)k);
     k_scatter_blocks<<<grid, 256, 0, s>>>(layer, serialized, static_cast<const uint32_t*>(c->mirror_dev),
-                                          reinterpret_cast<const int32_t*>(c->cnt) + at, (uint32_t)k,
+                                          reinterpret_cast<const int32_t*>(S.cnt) + at, (uint32_t)k,
                                           (uint32_t)c->vox_per_block, pool, updated_bits ? d_upd : nullptr, flags,
                                           layer == VBX_LAYER_ESDF ? c->tab.slot_has_esdf : nullptr);
     VBX_CUDA(c, cudaStreamSynchronize(s));  // the staging buffer is reused by the next chunk
@@ -237,7 +238,7 @@ int remove_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m);
 
 // Layer::removeAllBlocks (core/layer.h:164) of ONE layer; the other layer keeps its blocks
 int clear_layer(vbx_ctx* c, int layer) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   if (layer == VBX_LAYER_ESDF && !c->has_esdf) return VBX_OK;
   if (c->has_esdf && c->n_blocks) {
     // the layers share pool slots: remove this layer's block from every slot (slots that end up
@@ -275,7 +276,7 @@ int clear_layer(vbx_ctx* c, int layer) {
 
 int remove_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m) {
   if (m == 0) return VBX_OK;
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   if (int rc = refresh_host_mirror(c)) return rc;
   std::vector<int32_t> victims;
   for (uint64_t i = 0; i < m; ++i) {
@@ -374,7 +375,7 @@ __global__ void k_gather_blocks(const uint4* __restrict__ pool, const uint32_t* 
 
 int mirror_updated(vbx_ctx* c, int layer, int updated_mask, int clear_mask, int32_t* idx3, void* voxels,
                    uint8_t* updated_bits, uint64_t cap, uint64_t* n, int serialized) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   *n = 0;
   if (c->n_blocks == 0) return VBX_OK;
   if (int rc = refresh_host_mirror(c)) return rc;

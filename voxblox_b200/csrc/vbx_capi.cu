@@ -45,8 +45,8 @@ int refresh_host_mirror(vbx_ctx* c) {
   if (have < c->n_blocks) {
     c->host_slot_key.resize(c->n_blocks);
     VBX_CUDA(c, cudaMemcpyAsync(c->host_slot_key.data() + have, c->tab.slot_key + have,
-                                (c->n_blocks - have) * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
-    VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+                                (c->n_blocks - have) * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream_main));
+    VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
     for (size_t s = have; s < c->n_blocks; ++s) c->host_key2slot[c->host_slot_key[s]] = (int32_t)s;
   }
   return VBX_OK;
@@ -123,45 +123,6 @@ static int recover_async(vbx_ctx* c) {
   return first_rc;
 }
 
-void select_set(vbx_ctx* c, int k) {
-  const vbx_ctx::ScratchSet& S = c->set[k];
-  c->ray_p = S.ray_p;
-  c->ray_a = S.ray_a;
-  c->ray_c = S.ray_c;
-  c->ray_list = S.ray_list;
-  c->head_list = S.head_list;
-  c->tab.touched_list = S.touched_list;
-  c->cnt = S.cnt;
-  c->off = S.off;
-  c->d_state = S.d_state;
-  c->h_state = S.h_state;
-  c->d_xyz = S.d_xyz;
-  c->d_rgba = S.d_rgba;
-  c->pkeys[0] = S.pkeys0;
-  for (int i = 0; i < 2; ++i) {
-    c->ckeys[i] = S.ckeys[i];
-    c->cvals[i] = S.cvals[i];
-  }
-  c->sort_plan[1] = S.sort_plan1;
-  c->sort_status[1] = S.sort_status1;
-}
-
-void select_lane(vbx_ctx* c, int l) {
-  const vbx_ctx::FrontLane& F = c->lane[l];
-  c->big_list = F.big_list;
-  c->first_bits = F.first_bits;
-  c->order_scratch = F.order_scratch;
-  c->side_stream = F.side;
-  c->ev_fork = F.ev_fork;
-  c->ev_join = F.ev_join;
-  c->pkeys[1] = F.pkeys1;
-  c->pvals[0] = F.pvals[0];
-  c->pvals[1] = F.pvals[1];
-  c->sort_plan[0] = F.sort_plan0;
-  c->sort_status[0] = F.sort_status0;
-  c->scan_status = F.scan_status;
-}
-
 int drain_async(vbx_ctx* c) {
   for (int k = 0; k < c->sets_in_use; ++k) {
     vbx_ctx::ScratchSet& S = c->set[(c->async_seq + k) % c->sets_in_use];  // oldest submission first
@@ -169,12 +130,6 @@ int drain_async(vbx_ctx* c) {
     VBX_CUDA(c, cudaEventSynchronize(S.back_done));
     harvest_async(c, S);
   }
-  // synchronous calls use hand-off set 0 and front lane 0 on the main stream
-  select_set(c, 0);
-  select_lane(c, 0);
-  c->stream = c->stream_main;
-  c->apply_stream = nullptr;
-  c->sort_stream = nullptr;
   if (int rc = recover_async(c)) {
     if (!c->deferred_rc) return rc;
   }
@@ -192,36 +147,91 @@ static cudaError_t dmalloc(T** p, size_t count) {
   return cudaMalloc(reinterpret_cast<void**>(p), count * sizeof(T));
 }
 
-// k_bundle_order's tables for one front lane (vbx_order.cuh)
-int alloc_order_scratch(vbx_ctx* c, OrderScratch* g, uint32_t** big_list, uint32_t** first_bits) {
+// The device buffers of one hand-off set (its events are created by ensure_async).
+static int alloc_set(vbx_ctx* c, vbx_ctx::ScratchSet& S) {
   const size_t np = c->max_points;
-  std::memset(g, 0, sizeof(*g));
-  g->cap = (uint32_t)np;
-  // the bucket count after np insertions
-  uint32_t buckets = 1;
-  for (int k = 0; k < c->rehash.count && c->rehash.m[k] < np; ++k) buckets = c->rehash.n[k];
-  g->bucket_cap = buckets;
-  VBX_CUDA(c, dmalloc(&g->h, 2 * np));
-  VBX_CUDA(c, dmalloc(&g->tau, np));
-  VBX_CUDA(c, dmalloc(&g->tau2, np));
-  VBX_CUDA(c, dmalloc(&g->next, np));
-  VBX_CUDA(c, dmalloc(&g->bkt, np));
-  VBX_CUDA(c, dmalloc(&g->A, np));
-  VBX_CUDA(c, dmalloc(&g->bhead, (size_t)buckets));
-  VBX_CUDA(c, dmalloc(&g->head_of, 2 * np));
-  VBX_CUDA(c, dmalloc(&g->wp, 2 * (np / 32 + 2)));
-  VBX_CUDA(c, dmalloc(&g->cta_tot, 64));
-  VBX_CUDA(c, dmalloc(big_list, np / 256 + 2));
-  VBX_CUDA(c, dmalloc(first_bits, 2 * (np / 32 + 2)));
-  VBX_CUDA(c, cudaMemsetAsync(*first_bits, 0, 2 * (np / 32 + 2) * sizeof(uint32_t), c->stream_main));
+  VBX_CUDA(c, dmalloc(&S.d_xyz, 3 * np));
+  VBX_CUDA(c, dmalloc(&S.d_rgba, 4 * np));
+  VBX_CUDA(c, dmalloc(&S.pkeys0, np));
+  for (int i = 0; i < 2; ++i) {
+    VBX_CUDA(c, dmalloc(&S.ckeys[i], (size_t)c->max_updates));
+    VBX_CUDA(c, dmalloc(&S.cvals[i], (size_t)c->max_updates));
+  }
+  VBX_CUDA(c, dmalloc(&S.ray_p, np));
+  VBX_CUDA(c, dmalloc(&S.ray_a, np));
+  VBX_CUDA(c, dmalloc(&S.ray_c, np));
+  VBX_CUDA(c, dmalloc(&S.ray_list, np));
+  VBX_CUDA(c, dmalloc(&S.head_list, np));
+  VBX_CUDA(c, dmalloc(&S.touched_list, c->tab.touched_cap));
+  VBX_CUDA(c, dmalloc(&S.cnt, np + 1));
+  VBX_CUDA(c, dmalloc(&S.off, np + 1));
+  VBX_CUDA(c, dmalloc(&S.sort_plan1, 1));
+  VBX_CUDA(c, dmalloc(&S.sort_status1, (size_t)4 * c->sort_tiles_cap[1] * kRadix));
+  VBX_CUDA(c, dmalloc(&S.d_state, 1));
+  VBX_CUDA(c, cudaMallocHost(reinterpret_cast<void**>(&S.h_state), sizeof(ScanState)));
   return VBX_OK;
 }
-void free_order_scratch(OrderScratch* g, uint32_t* big_list, uint32_t* first_bits) {
-  void* ptrs[] = {g->h, g->tau, g->tau2, g->next, g->bkt, g->A, g->bhead, g->head_of, g->wp, g->cta_tot, big_list, first_bits};
+
+static void free_set(vbx_ctx::ScratchSet& S) {
+  void* ptrs[] = {S.d_xyz, S.d_rgba, S.pkeys0, S.ckeys[0], S.ckeys[1], S.cvals[0], S.cvals[1], S.ray_p, S.ray_a,
+                  S.ray_c, S.ray_list, S.head_list, S.touched_list, S.cnt, S.off, S.sort_plan1, S.sort_status1, S.d_state};
   for (void* p : ptrs) {
     if (p) cudaFree(p);
   }
-  std::memset(g, 0, sizeof(*g));
+  if (S.h_state) cudaFreeHost(S.h_state);
+  cudaEvent_t evs[] = {S.copy_done, S.front_done, S.walked, S.sorted, S.back_done, S.applied, S.front_start};
+  for (cudaEvent_t e : evs) {
+    if (e) cudaEventDestroy(e);
+  }
+}
+
+// The device buffers of one front lane, k_bundle_order's tables (vbx_order.cuh) among them (its streams
+// and events are created by vbx_create / ensure_async).
+static int alloc_lane(vbx_ctx* c, vbx_ctx::FrontLane& F) {
+  const size_t np = c->max_points;
+  VBX_CUDA(c, dmalloc(&F.pkeys1, np));
+  VBX_CUDA(c, dmalloc(&F.pvals[0], np));
+  VBX_CUDA(c, dmalloc(&F.pvals[1], np));
+  VBX_CUDA(c, dmalloc(&F.sort_plan0, 1));
+  VBX_CUDA(c, dmalloc(&F.sort_status0, (size_t)8 * c->sort_tiles_cap[0] * kRadix));
+  VBX_CUDA(c, dmalloc(&F.scan_status, (np + 1) / kScanTile + 4));
+  OrderScratch& g = F.order_scratch;
+  g.cap = (uint32_t)np;
+  // the bucket count after np insertions
+  uint32_t buckets = 1;
+  for (int k = 0; k < c->rehash.count && c->rehash.m[k] < np; ++k) buckets = c->rehash.n[k];
+  g.bucket_cap = buckets;
+  VBX_CUDA(c, dmalloc(&g.h, 2 * np));
+  VBX_CUDA(c, dmalloc(&g.tau, np));
+  VBX_CUDA(c, dmalloc(&g.tau2, np));
+  VBX_CUDA(c, dmalloc(&g.next, np));
+  VBX_CUDA(c, dmalloc(&g.bkt, np));
+  VBX_CUDA(c, dmalloc(&g.A, np));
+  VBX_CUDA(c, dmalloc(&g.bhead, (size_t)buckets));
+  VBX_CUDA(c, dmalloc(&g.head_of, 2 * np));
+  VBX_CUDA(c, dmalloc(&g.wp, 2 * (np / 32 + 2)));
+  VBX_CUDA(c, dmalloc(&g.cta_tot, 64));
+  VBX_CUDA(c, dmalloc(&F.big_list, np / 256 + 2));
+  VBX_CUDA(c, dmalloc(&F.first_bits, 2 * (np / 32 + 2)));
+  VBX_CUDA(c, cudaMemsetAsync(F.first_bits, 0, 2 * (np / 32 + 2) * sizeof(uint32_t), c->stream_main));
+  return VBX_OK;
+}
+
+static void free_lane(vbx_ctx::FrontLane& F) {
+  const OrderScratch& g = F.order_scratch;
+  void* ptrs[] = {F.pkeys1, F.pvals[0], F.pvals[1], F.sort_plan0, F.sort_status0, F.scan_status, F.big_list, F.first_bits,
+                  g.h,      g.tau,      g.tau2,     g.next,       g.bkt,          g.A,           g.bhead,    g.head_of,
+                  g.wp,     g.cta_tot};
+  for (void* p : ptrs) {
+    if (p) cudaFree(p);
+  }
+  if (F.side) {
+    cudaStreamSynchronize(F.side);
+    cudaStreamDestroy(F.side);
+  }
+  if (F.ev_fork) cudaEventDestroy(F.ev_fork);
+  if (F.ev_join) cudaEventDestroy(F.ev_join);
+  if (F.stream) cudaStreamDestroy(F.stream);
 }
 
 }  // namespace vbx
@@ -311,7 +321,6 @@ int vbx_create(const vbx_tsdf_config* cfg, float voxel_size, int voxels_per_side
   CK(cudaStreamCreateWithPriority(&c->stream_main, cudaStreamNonBlocking, prio_hi));
   CK(cudaStreamCreateWithFlags(&c->stream_c, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&c->stream_c2, cudaStreamNonBlocking));
-  c->stream = c->stream_main;
   CK(cudaEventCreate(&c->ev0));
   CK(cudaEventCreate(&c->ev1));
   CK(cudaEventCreate(&c->tev0));
@@ -331,35 +340,29 @@ int vbx_create(const vbx_tsdf_config* cfg, float voxel_size, int voxels_per_side
   // ids lost to first-touch races stay unused (vbx_hash.cuh); (id, voxel) must fit a 32-bit record key
   t.touched_cap = (uint32_t)std::min<uint64_t>((uint64_t)o.max_blocks + 65536u, (0xffffffffull >> (3 * c->L)) - 1);
   t.vox_per_block = c->vox_per_block;
-  CK(dmalloc(&t.touched_list, t.touched_cap));
   CK(dmalloc(&t.slot_key, o.max_blocks));
   CK(dmalloc(&t.slot_updated, o.max_blocks));
   CK(dmalloc(&t.slot_esdf_updated, o.max_blocks));
   CK(dmalloc(&t.slot_has_esdf, o.max_blocks));
   CK(dmalloc(&t.tsdf, (size_t)o.max_blocks * c->vox_per_block));
-  CK(cudaMemsetAsync(t.hkeys, 0xff, (size_t)hcap * sizeof(uint64_t), c->stream));
-  CK(cudaMemsetAsync(t.hslot, 0xff, (size_t)hcap * sizeof(int32_t), c->stream));
-  CK(cudaMemsetAsync(t.htouch, 0, (size_t)hcap * sizeof(unsigned long long), c->stream));
-  CK(cudaMemsetAsync(t.slot_updated, 0, o.max_blocks, c->stream));
-  CK(cudaMemsetAsync(t.slot_esdf_updated, 0, o.max_blocks, c->stream));
-  CK(cudaMemsetAsync(t.slot_has_esdf, 0, o.max_blocks, c->stream));
+  CK(cudaMemsetAsync(t.hkeys, 0xff, (size_t)hcap * sizeof(uint64_t), c->stream_main));
+  CK(cudaMemsetAsync(t.hslot, 0xff, (size_t)hcap * sizeof(int32_t), c->stream_main));
+  CK(cudaMemsetAsync(t.htouch, 0, (size_t)hcap * sizeof(unsigned long long), c->stream_main));
+  CK(cudaMemsetAsync(t.slot_updated, 0, o.max_blocks, c->stream_main));
+  CK(cudaMemsetAsync(t.slot_esdf_updated, 0, o.max_blocks, c->stream_main));
+  CK(cudaMemsetAsync(t.slot_has_esdf, 0, o.max_blocks, c->stream_main));
   // new Block: voxels default-constructed = all zero bytes (core/voxel.h:12-16)
-  CK(cudaMemsetAsync(t.tsdf, 0, (size_t)o.max_blocks * c->vox_per_block * sizeof(TsdfVoxel), c->stream));
+  CK(cudaMemsetAsync(t.tsdf, 0, (size_t)o.max_blocks * c->vox_per_block * sizeof(TsdfVoxel), c->stream_main));
   const size_t np = c->max_points;
-  CK(dmalloc(&c->d_xyz, 3 * np));
-  CK(dmalloc(&c->d_rgba, 4 * np));
-  for (int i = 0; i < 2; ++i) {
-    CK(dmalloc(&c->pkeys[i], np));
-    CK(dmalloc(&c->pvals[i], np));
-    CK(dmalloc(&c->ckeys[i], (size_t)c->max_updates));
-    CK(dmalloc(&c->cvals[i], (size_t)c->max_updates));
-  }
+  c->sort_tiles_cap[0] = (uint32_t)((np + kSortTile - 1) / kSortTile);
+  c->sort_tiles_cap[1] = (uint32_t)((c->max_updates + kSortTile - 1) / kSortTile);
+  if (int rc = init_bundle_order(c)) return rc;
+  // hand-off set 0 and front lane 0 serve the synchronous calls; ensure_async allocates the others
+  if (int rc = alloc_set(c, c->set[0])) return rc;
+  if (int rc = alloc_lane(c, c->lane[0])) return rc;
+  CK(cudaMemsetAsync(c->set[0].d_state, 0, sizeof(ScanState), c->stream_main));
   CK(dmalloc(&c->order, np));
   CK(dmalloc(&c->order_inv, np));
-  CK(dmalloc(&c->ray_list, np));
-  if (int rc = init_bundle_order(c)) return rc;
-  CK(dmalloc(&c->head_list, np));
-  if (int rc = alloc_order_scratch(c, &c->order_scratch, &c->big_list, &c->first_bits)) return rc;
   for (int l = 0; l < vbx_ctx::kLanes; ++l) {
     CK(cudaStreamCreateWithPriority(&c->lane[l].side, cudaStreamNonBlocking, prio_lo));
     CK(cudaEventCreateWithFlags(&c->lane[l].ev_fork, cudaEventDisableTiming));
@@ -372,68 +375,15 @@ int vbx_create(const vbx_tsdf_config* cfg, float voxel_size, int voxels_per_side
   CK(dmalloc(&c->verify_start, (size_t)(c->max_updates / 32 + 1)));
   CK(dmalloc(&c->rec_sdf, (size_t)c->max_updates));
   CK(dmalloc(&c->rec_w, (size_t)c->max_updates));
-  CK(dmalloc(&c->ray_p, np));
-  CK(dmalloc(&c->ray_c, np));
-  CK(dmalloc(&c->ray_a, np));
-  CK(dmalloc(&c->cnt, np + 1));
-  CK(dmalloc(&c->off, np + 1));
-  {
-    // own sort / scan state
-    c->sort_tiles_cap[0] = (uint32_t)((np + kSortTile - 1) / kSortTile);
-    c->sort_tiles_cap[1] = (uint32_t)((c->max_updates + kSortTile - 1) / kSortTile);
-    for (int i = 0; i < 2; ++i) {
-      CK(dmalloc(&c->sort_plan[i], 1));
-      const size_t words = (size_t)(i == 0 ? 8 : 4) * c->sort_tiles_cap[i] * kRadix;
-      CK(dmalloc(&c->sort_status[i], words));
-    }
-    CK(dmalloc(&c->scan_status, (np + 1) / kScanTile + 4));
-  }
   CK(dmalloc(&c->set_start, 1u << 20));
   CK(dmalloc(&c->set_observed, 1u << 20));
-  CK(cudaMemsetAsync(c->set_start, 0, sizeof(unsigned long long) << 20, c->stream));
-  CK(cudaMemsetAsync(c->set_observed, 0, sizeof(unsigned long long) << 20, c->stream));
-  CK(dmalloc(&c->d_state, 1));
-  CK(cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), c->stream));
-  CK(cudaMallocHost(reinterpret_cast<void**>(&c->h_state), sizeof(ScanState)));
+  CK(cudaMemsetAsync(c->set_start, 0, sizeof(unsigned long long) << 20, c->stream_main));
+  CK(cudaMemsetAsync(c->set_observed, 0, sizeof(unsigned long long) << 20, c->stream_main));
   CK(dmalloc(&c->d_nblocks, 2));
-  CK(cudaMemsetAsync(c->d_nblocks, 0, 2 * sizeof(uint32_t), c->stream));
+  CK(cudaMemsetAsync(c->d_nblocks, 0, 2 * sizeof(uint32_t), c->stream_main));
   CK(dmalloc(&c->d_hold, 1));
-  CK(cudaMemsetAsync(c->d_hold, 0, sizeof(uint32_t), c->stream));
-  {
-    // hand-off set 0 / front lane 0 are the buffers above; the others are allocated by ensure_async
-    vbx_ctx::ScratchSet& a = c->set[0];
-    a.ray_p = c->ray_p;
-    a.ray_a = c->ray_a;
-    a.ray_c = c->ray_c;
-    a.ray_list = c->ray_list;
-    a.head_list = c->head_list;
-    a.touched_list = c->tab.touched_list;
-    a.cnt = c->cnt;
-    a.off = c->off;
-    a.d_state = c->d_state;
-    a.h_state = c->h_state;
-    a.d_xyz = c->d_xyz;
-    a.d_rgba = c->d_rgba;
-    a.pkeys0 = c->pkeys[0];
-    for (int i = 0; i < 2; ++i) {
-      a.ckeys[i] = c->ckeys[i];
-      a.cvals[i] = c->cvals[i];
-    }
-    a.sort_plan1 = c->sort_plan[1];
-    a.sort_status1 = c->sort_status[1];
-    vbx_ctx::FrontLane& f = c->lane[0];
-    f.pkeys1 = c->pkeys[1];
-    f.pvals[0] = c->pvals[0];
-    f.pvals[1] = c->pvals[1];
-    f.sort_plan0 = c->sort_plan[0];
-    f.sort_status0 = c->sort_status[0];
-    f.scan_status = c->scan_status;
-    f.big_list = c->big_list;
-    f.first_bits = c->first_bits;
-    f.order_scratch = c->order_scratch;
-    select_lane(c, 0);
-  }
-  CK(cudaStreamSynchronize(c->stream));
+  CK(cudaMemsetAsync(c->d_hold, 0, sizeof(uint32_t), c->stream_main));
+  CK(cudaStreamSynchronize(c->stream_main));
 #undef CK
   return VBX_OK;
 }
@@ -441,7 +391,7 @@ int vbx_create(const vbx_tsdf_config* cfg, float voxel_size, int voxels_per_side
 }  // extern "C" (reopened below)
 
 namespace vbx {
-// First asynchronous submission: the remaining hand-off sets, the second front lane, streams, events.
+// First asynchronous submission: the remaining hand-off sets and front lanes, streams, events.
 int ensure_async(vbx_ctx* c) {
   if (c->async_ready) return VBX_OK;
 #define CK(expr)                                           \
@@ -451,7 +401,6 @@ int ensure_async(vbx_ctx* c) {
   } while (0)
   if (const char* e = std::getenv("VBX_ASYNC_SETS")) c->sets_in_use = std::max(2, std::min(std::atoi(e), (int)vbx_ctx::kSets));
   if (const char* e = std::getenv("VBX_ASYNC_LANES")) c->lanes_in_use = std::max(1, std::min(std::atoi(e), (int)vbx_ctx::kLanes));
-  const size_t np = c->max_points;
   CK(cudaStreamCreateWithFlags(&c->stream_h, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithPriority(&c->stream_e, cudaStreamNonBlocking, std::min(c->prio_lo, c->prio_hi + 1)));
   for (int i = 0; i < vbx_ctx::kSortStreams; ++i) {
@@ -460,14 +409,9 @@ int ensure_async(vbx_ctx* c) {
   for (int l = 0; l < c->lanes_in_use; ++l) {
     vbx_ctx::FrontLane& F = c->lane[l];
     CK(cudaStreamCreateWithPriority(&F.stream, cudaStreamNonBlocking, c->prio_lo));
-    if (l == 0) continue;
-    CK(dmalloc(&F.pkeys1, np));
-    CK(dmalloc(&F.pvals[0], np));
-    CK(dmalloc(&F.pvals[1], np));
-    CK(dmalloc(&F.sort_plan0, 1));
-    CK(dmalloc(&F.sort_status0, (size_t)8 * c->sort_tiles_cap[0] * kRadix));
-    CK(dmalloc(&F.scan_status, (np + 1) / kScanTile + 4));
-    if (int rc = alloc_order_scratch(c, &F.order_scratch, &F.big_list, &F.first_bits)) return rc;
+    if (l > 0) {
+      if (int rc = alloc_lane(c, F)) return rc;
+    }
   }
   // diagnostic: with VBX_ASYNC_TIMELINE set the hand-off events keep timestamps (vbx_debug_async_timeline)
   c->timeline = std::getenv("VBX_ASYNC_TIMELINE") != nullptr;
@@ -485,26 +429,9 @@ int ensure_async(vbx_ctx* c) {
     CK(cudaEventCreateWithFlags(&S.back_done, evf));
     CK(cudaEventCreateWithFlags(&S.applied, evf));
     if (c->timeline) CK(cudaEventCreate(&S.front_start));
-    if (k == 0) continue;
-    CK(dmalloc(&S.ray_p, np));
-    CK(dmalloc(&S.ray_a, np));
-    CK(dmalloc(&S.ray_c, np));
-    CK(dmalloc(&S.ray_list, np));
-    CK(dmalloc(&S.head_list, np));
-    CK(dmalloc(&S.touched_list, c->tab.touched_cap));
-    CK(dmalloc(&S.cnt, np + 1));
-    CK(dmalloc(&S.off, np + 1));
-    CK(dmalloc(&S.d_state, 1));
-    CK(cudaMallocHost(reinterpret_cast<void**>(&S.h_state), sizeof(ScanState)));
-    CK(dmalloc(&S.d_xyz, 3 * np));
-    CK(dmalloc(&S.d_rgba, 4 * np));
-    CK(dmalloc(&S.pkeys0, np));
-    for (int i = 0; i < 2; ++i) {
-      CK(dmalloc(&S.ckeys[i], (size_t)c->max_updates));
-      CK(dmalloc(&S.cvals[i], (size_t)c->max_updates));
+    if (k > 0) {
+      if (int rc = alloc_set(c, S)) return rc;
     }
-    CK(dmalloc(&S.sort_plan1, 1));
-    CK(dmalloc(&S.sort_status1, (size_t)4 * c->sort_tiles_cap[1] * kRadix));
   }
 #undef CK
   c->async_ready = true;
@@ -528,64 +455,21 @@ void vbx_destroy(vbx_ctx* c) {
   for (int l = 0; l < vbx_ctx::kLanes; ++l) {
     if (c->lane[l].stream) cudaStreamSynchronize(c->lane[l].stream);
   }
-  // restore the aliases of hand-off set 0 / lane 0 before freeing
-  select_set(c, 0);
-  select_lane(c, 0);
-  c->stream = c->stream_main;
   esdf_destroy(c);
   mesh_destroy(c);
   icp_destroy(c);
   Tables& t = c->tab;
-  void* ptrs[] = {t.hkeys,        t.hslot,       t.htouch, t.new_list, t.touched_list,
-                  t.slot_key,     t.slot_updated, t.slot_esdf_updated, t.slot_has_esdf, t.tsdf, c->d_xyz,
-                  c->d_rgba,      c->pkeys[0],   c->pkeys[1],    c->pvals[0],   c->pvals[1], c->ckeys[0],
-                  c->ckeys[1],    c->cvals[0],   c->cvals[1],    c->order,      c->ray_p,    c->ray_c,
-                  c->cnt,         c->off,        c->set_start,  c->set_observed, c->d_state,
-                  c->ray_list,    c->head_list,  c->long_list,  c->ray_a,      c->sort_plan[0], c->sort_plan[1],
-                  c->sort_status[0], c->sort_status[1], c->scan_status, c->long_end, c->long_state,
-                  c->verify_run,  c->verify_start, c->rec_sdf, c->rec_w, c->d_nblocks, c->order_inv, c->d_hold};
+  void* ptrs[] = {t.hkeys, t.hslot, t.htouch, t.new_list, t.slot_key, t.slot_updated, t.slot_esdf_updated,
+                  t.slot_has_esdf, t.tsdf, c->order, c->order_inv, c->set_start, c->set_observed, c->long_list,
+                  c->long_end, c->long_state, c->verify_run, c->verify_start, c->rec_sdf, c->rec_w, c->d_nblocks, c->d_hold};
   for (void* p : ptrs) {
     if (p) cudaFree(p);
   }
-  if (c->h_state) cudaFreeHost(c->h_state);
   if (c->mirror_dev) cudaFree(c->mirror_dev);
   if (c->mirror_host) cudaFreeHost(c->mirror_host);
   if (c->mirror_slots) cudaFree(c->mirror_slots);
-  for (int k = 0; k < vbx_ctx::kSets; ++k) {
-    vbx_ctx::ScratchSet& S = c->set[k];
-    if (k > 0) {
-      void* sp[] = {S.ray_p, S.ray_a, S.ray_c, S.ray_list, S.head_list, S.touched_list, S.cnt, S.off, S.d_state, S.d_xyz, S.d_rgba, S.pkeys0,
-                    S.ckeys[0], S.ckeys[1], S.cvals[0], S.cvals[1], S.sort_plan1, S.sort_status1};
-      for (void* p : sp) {
-        if (p) cudaFree(p);
-      }
-      if (S.h_state) cudaFreeHost(S.h_state);
-    }
-    if (S.copy_done) cudaEventDestroy(S.copy_done);
-    if (S.front_done) cudaEventDestroy(S.front_done);
-    if (S.walked) cudaEventDestroy(S.walked);
-    if (S.sorted) cudaEventDestroy(S.sorted);
-    if (S.back_done) cudaEventDestroy(S.back_done);
-    if (S.applied) cudaEventDestroy(S.applied);
-    if (S.front_start) cudaEventDestroy(S.front_start);
-  }
-  for (int l = 0; l < vbx_ctx::kLanes; ++l) {
-    vbx_ctx::FrontLane& F = c->lane[l];
-    if (l > 0) {
-      void* fp[] = {F.pkeys1, F.pvals[0], F.pvals[1], F.sort_plan0, F.sort_status0, F.scan_status};
-      for (void* p : fp) {
-        if (p) cudaFree(p);
-      }
-    }
-    free_order_scratch(&F.order_scratch, F.big_list, F.first_bits);
-    if (F.side) {
-      cudaStreamSynchronize(F.side);
-      cudaStreamDestroy(F.side);
-    }
-    if (F.ev_fork) cudaEventDestroy(F.ev_fork);
-    if (F.ev_join) cudaEventDestroy(F.ev_join);
-    if (F.stream) cudaStreamDestroy(F.stream);
-  }
+  for (vbx_ctx::ScratchSet& S : c->set) free_set(S);
+  for (vbx_ctx::FrontLane& F : c->lane) free_lane(F);
   if (c->timeline_ref) cudaEventDestroy(c->timeline_ref);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -626,10 +510,10 @@ int vbx_tsdf_integrate(vbx_ctx* c, int kind, const float q[4], const float t[3],
   VBX_CUDA(c, cudaSetDevice(c->device));
   VBX_DRAIN(c);
   if (n) {
-    VBX_CUDA(c, cudaMemcpyAsync(c->d_xyz, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    VBX_CUDA(c, cudaMemcpyAsync(c->d_rgba, rgba, n * 4, cudaMemcpyHostToDevice, c->stream));
+    VBX_CUDA(c, cudaMemcpyAsync(c->set[0].d_xyz, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream_main));
+    VBX_CUDA(c, cudaMemcpyAsync(c->set[0].d_rgba, rgba, n * 4, cudaMemcpyHostToDevice, c->stream_main));
   }
-  return integrate_device(c, kind, q, t, c->d_xyz, c->d_rgba, n, freespace);
+  return integrate_device(c, kind, q, t, c->set[0].d_xyz, c->set[0].d_rgba, n, freespace);
 }
 
 int vbx_tsdf_integrate_async(vbx_ctx* c, int kind, const float q[4], const float t[3], const float* xyz,
@@ -731,9 +615,9 @@ int vbx_host_copy_ms(vbx_ctx* c, const void* src, size_t bytes, float* ms) {
   if (bytes > (size_t)c->max_points * 12) return fail(c, VBX_E_CAPACITY, "copy larger than the staging buffer");
   VBX_CUDA(c, cudaSetDevice(c->device));
   VBX_DRAIN(c);
-  VBX_CUDA(c, cudaEventRecord(c->tev0, c->stream));
-  VBX_CUDA(c, cudaMemcpyAsync(c->d_xyz, src, bytes, cudaMemcpyHostToDevice, c->stream));
-  VBX_CUDA(c, cudaEventRecord(c->tev1, c->stream));
+  VBX_CUDA(c, cudaEventRecord(c->tev0, c->stream_main));
+  VBX_CUDA(c, cudaMemcpyAsync(c->set[0].d_xyz, src, bytes, cudaMemcpyHostToDevice, c->stream_main));
+  VBX_CUDA(c, cudaEventRecord(c->tev1, c->stream_main));
   VBX_CUDA(c, cudaEventSynchronize(c->tev1));
   VBX_CUDA(c, cudaEventElapsedTime(ms, c->tev0, c->tev1));
   return VBX_OK;
@@ -743,7 +627,7 @@ int vbx_timer_start(vbx_ctx* c) {
   if (!c) return VBX_E_INVALID;
   VBX_CUDA(c, cudaSetDevice(c->device));
   VBX_DRAIN(c);
-  VBX_CUDA(c, cudaEventRecord(c->tev0, c->stream));
+  VBX_CUDA(c, cudaEventRecord(c->tev0, c->stream_main));
   return VBX_OK;
 }
 
@@ -751,7 +635,7 @@ int vbx_timer_stop_ms(vbx_ctx* c, float* ms) {
   if (!c || !ms) return VBX_E_INVALID;
   VBX_CUDA(c, cudaSetDevice(c->device));
   VBX_DRAIN(c);
-  VBX_CUDA(c, cudaEventRecord(c->tev1, c->stream));
+  VBX_CUDA(c, cudaEventRecord(c->tev1, c->stream_main));
   VBX_CUDA(c, cudaEventSynchronize(c->tev1));
   VBX_CUDA(c, cudaEventElapsedTime(ms, c->tev0, c->tev1));
   return VBX_OK;
@@ -787,12 +671,12 @@ static int fetch_flags(vbx_ctx* c, int layer, std::vector<uint8_t>* upd, std::ve
   has->assign(c->n_blocks, 1);
   if (c->n_blocks == 0) return VBX_OK;
   const uint8_t* src = (layer == VBX_LAYER_TSDF) ? c->tab.slot_updated : c->tab.slot_esdf_updated;
-  VBX_CUDA(c, cudaMemcpyAsync(upd->data(), src, c->n_blocks, cudaMemcpyDeviceToHost, c->stream));
+  VBX_CUDA(c, cudaMemcpyAsync(upd->data(), src, c->n_blocks, cudaMemcpyDeviceToHost, c->stream_main));
   if (layer == VBX_LAYER_ESDF) {
     VBX_CUDA(c, cudaMemcpyAsync(has->data(), c->tab.slot_has_esdf, c->n_blocks, cudaMemcpyDeviceToHost,
-                                c->stream));
+                                c->stream_main));
   }
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   for (uint32_t s = 0; s < c->n_blocks; ++s) {
     if (layer == VBX_LAYER_TSDF && ((*upd)[s] & kSlotNoTsdf)) (*has)[s] = 0;
     (*upd)[s] &= 0x07;  // kSlotNoTsdf / kEsdfPending / the mirror mark are internal
@@ -875,10 +759,10 @@ int vbx_download_blocks(vbx_ctx* c, int layer, const int32_t* idx3, uint64_t m, 
     auto it = c->host_key2slot.find(pack3(idx3[3 * i], idx3[3 * i + 1], idx3[3 * i + 2]));
     if (it == c->host_key2slot.end() || !has[it->second]) return fail(c, VBX_E_NOT_FOUND, "block not allocated");
     VBX_CUDA(c, cudaMemcpyAsync(static_cast<char*>(voxels) + i * bbytes, pool + (size_t)it->second * bbytes,
-                                bbytes, cudaMemcpyDeviceToHost, c->stream));
+                                bbytes, cudaMemcpyDeviceToHost, c->stream_main));
     if (updated_bits) updated_bits[i] = upd[it->second];
   }
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   return VBX_OK;
 }
 
@@ -917,11 +801,11 @@ int vbx_clear_updated(vbx_ctx* c, int layer, int updated_mask) {
   if (c->n_blocks == 0) return VBX_OK;
   std::vector<uint8_t> upd(c->n_blocks);
   uint8_t* dst = (layer == VBX_LAYER_TSDF) ? c->tab.slot_updated : c->tab.slot_esdf_updated;
-  VBX_CUDA(c, cudaMemcpyAsync(upd.data(), dst, c->n_blocks, cudaMemcpyDeviceToHost, c->stream));
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaMemcpyAsync(upd.data(), dst, c->n_blocks, cudaMemcpyDeviceToHost, c->stream_main));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   for (uint8_t& u : upd) u &= (uint8_t)(~updated_mask | 0x80);  // bit 7 is the engine's own (kSlotNoTsdf / kEsdfPending)
-  VBX_CUDA(c, cudaMemcpyAsync(dst, upd.data(), c->n_blocks, cudaMemcpyHostToDevice, c->stream));
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaMemcpyAsync(dst, upd.data(), c->n_blocks, cudaMemcpyHostToDevice, c->stream_main));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   return VBX_OK;
 }
 

@@ -102,7 +102,8 @@ struct Tables {
   uint32_t max_blocks;
   uint32_t vox_per_block;
   uint32_t* new_list;     // [max_blocks] hash positions created by this call
-  uint32_t* touched_list; // [touched_cap] touched id -> hash position (0xffffffff: unused id); hand-off set private
+  uint32_t* touched_list; // [touched_cap] touched id -> hash position (0xffffffff: unused id); null in vbx_ctx::tab,
+                          // the launch code passes a copy that points at the hand-off set's own list
   uint32_t touched_cap;
   uint64_t* slot_key;     // [max_blocks] packed block index per pool slot
   uint8_t* slot_updated;  // [max_blocks] TSDF Block::updated() bits
@@ -139,7 +140,6 @@ __host__ __device__ inline uint32_t hash64(uint64_t k) {
 
 struct vbx_ctx {
   int device = 0;
-  cudaStream_t stream = nullptr;      // the stream the next launch goes to (main, or a pipeline stage's stream while one is enqueued)
   cudaStream_t stream_main = nullptr; // back halves, ESDF, block management, synchronous calls
   cudaStream_t stream_c = nullptr;    // host-to-device cloud copies of asynchronously submitted scans
   cudaStream_t stream_c2 = nullptr;   // ... alternating with this one
@@ -160,19 +160,8 @@ struct vbx_ctx {
   cudaEvent_t timeline_ref = nullptr;
   uint32_t bundle_hint = 0;         // bundles (the larger of the two maps) of the most recent Merged scan whose counters reached the host
   uint64_t record_hint = 1u << 20;  // update records of the most recent scan whose count reached the host: sizes the record sort's grid
-  float* d_xyz = nullptr;
-  uint8_t* d_rgba = nullptr;
-  uint64_t* pkeys[2] = {nullptr, nullptr};
-  uint32_t* pvals[2] = {nullptr, nullptr};
-  uint32_t* order = nullptr;
-  uint32_t* order_inv = nullptr;           // [max_points] inverse of `order` ("sorted" integration order)
-  uint32_t* ray_list = nullptr;            // [max_points] Merged: ray slot (rank in the reference's bundle order) -> head
-  uint32_t* head_list = nullptr;           // [max_points] bundle heads, unordered (hand-off set private)
-  uint32_t* big_list = nullptr;            // [max_points / 256 + 1] ids of the big bundles (front-lane private)
-  cudaStream_t side_stream = nullptr;      // k_bundle_order runs here, beside k_merge (front-lane private)
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  uint32_t* first_bits = nullptr;          // [2][max_points / 32 + 1] first-occurrence bitmaps (front-lane private)
-  vbx::OrderScratch order_scratch{};         // k_bundle_order's global tables (front-lane private)
+  uint32_t* order = nullptr;               // [max_points] "sorted" integration order (synchronous calls only)
+  uint32_t* order_inv = nullptr;           // [max_points] inverse of `order`
   vbx::RehashSchedule rehash{};            // libstdc++'s unordered_map growth schedule (vbx_create)
   size_t order_smem_bytes = 0;             // dynamic shared memory of k_bundle_order
   unsigned long long* long_list = nullptr; // [max_updates / 32 + 1] starts of long voxel runs
@@ -182,24 +171,11 @@ struct vbx_ctx {
   unsigned long long* verify_start = nullptr;
   float* rec_sdf = nullptr;                // [max_updates] per sorted record
   float* rec_w = nullptr;
-  float4* ray_p = nullptr;    // point_G.xyz, flags (bit 0: clearing ray)
-  float4* ray_a = nullptr;    // point_G - origin, |point_G - origin|
-  uint2* ray_c = nullptr;     // colour, weight bits
-  uint32_t* cnt = nullptr;    // [max_points + 1]
-  uint32_t* off = nullptr;    // [max_points + 1]
-  uint32_t* ckeys[2] = {nullptr, nullptr};
-  uint32_t* cvals[2] = {nullptr, nullptr};
-  // the engine's own radix sort / scan (vbx_sort.cuh): [0] point keys, [1] update records
-  vbx::SortPlan* sort_plan[2] = {nullptr, nullptr};
-  uint32_t* sort_status[2] = {nullptr, nullptr};
-  uint32_t sort_tiles_cap[2] = {0, 0};
-  uint32_t* scan_status = nullptr;
+  uint32_t sort_tiles_cap[2] = {0, 0};  // tiles of the engine's radix sort (vbx_sort.cuh): [0] point keys, [1] update records
   unsigned long long* set_start = nullptr;  // Fast integrator approximate sets
   unsigned long long* set_observed = nullptr;
   uint32_t set_epoch = 1;
   int64_t fast_reset_counter = 0;
-  vbx::ScanState* d_state = nullptr;
-  vbx::ScanState* h_state = nullptr;  // pinned
   uint32_t epoch = 0;                 // call id for touch marks
   uint32_t n_blocks = 0;              // pool slots in use (host copy, exact after a drain)
   uint32_t* d_nblocks = nullptr;      // [2] device copy, ping-pong: k_assign reads [nb_cur], writes [nb_cur ^ 1]
@@ -208,27 +184,28 @@ struct vbx_ctx {
   // separate streams -- front half (keys, bundle sort, bundle fold, offsets; does not touch the map)
   // on one of kLanes front streams, ray walk + block creation + record sort on stream_e, apply on
   // the main stream -- so up to kSets scans are in flight, each owning one set of hand-off
-  // buffers.  Map-touching stages run in submission order.  Set 0 / lane 0 are the buffers the
-  // synchronous calls use; the others are allocated on the first asynchronous submission.
+  // buffers.  Map-touching stages run in submission order.  The launch code takes the set and the
+  // lane it works on as arguments.  Synchronous calls name set 0 and lane 0 and run on the main
+  // stream; the other sets and lanes are allocated on the first asynchronous submission.
   static constexpr int kSets = 16, kLanes = 8, kSortStreams = 2;  // upper bounds
   int sets_in_use = 10, lanes_in_use = 6;  // (tuning aids: VBX_ASYNC_SETS, VBX_ASYNC_LANES)
   struct ScratchSet {
-    float4* ray_p = nullptr;
-    float4* ray_a = nullptr;
-    uint2* ray_c = nullptr;
-    uint32_t* ray_list = nullptr;
+    float4* ray_p = nullptr;  // point_G.xyz, flags (bit 0: clearing ray)
+    float4* ray_a = nullptr;  // point_G - origin, |point_G - origin|
+    uint2* ray_c = nullptr;   // colour, weight bits
+    uint32_t* ray_list = nullptr;    // Merged: ray slot (rank in the reference's bundle order) -> head
     uint32_t* head_list = nullptr;   // bundle id -> sorted position of its head (read again by the ray walk)
-    uint32_t* touched_list = nullptr;  // touched id -> hash position (written by the walk, read by the apply)
-    uint32_t* cnt = nullptr;
-    uint32_t* off = nullptr;
+    uint32_t* touched_list = nullptr;  // [touched_cap] touched id -> hash position (written by the walk, read by the apply)
+    uint32_t* cnt = nullptr;  // [max_points + 1]
+    uint32_t* off = nullptr;  // [max_points + 1]
     vbx::ScanState* d_state = nullptr;
-    vbx::ScanState* h_state = nullptr;
+    vbx::ScanState* h_state = nullptr;  // pinned
     float* d_xyz = nullptr;
     uint8_t* d_rgba = nullptr;
     uint64_t* pkeys0 = nullptr;  // sorted bundle keys (read again by the ray walk)
-    uint32_t* ckeys[2] = {nullptr, nullptr};  // update records (written by the walk, read by apply)
+    uint32_t* ckeys[2] = {nullptr, nullptr};  // [max_updates] update records (written by the walk, read by apply)
     uint32_t* cvals[2] = {nullptr, nullptr};
-    vbx::SortPlan* sort_plan1 = nullptr;
+    vbx::SortPlan* sort_plan1 = nullptr;      // the update-record sort (vbx_sort.cuh)
     uint32_t* sort_status1 = nullptr;
     cudaEvent_t copy_done = nullptr, front_done = nullptr, walked = nullptr, sorted = nullptr, back_done = nullptr;
     cudaEvent_t applied = nullptr;      // the apply kernels are done (the status read-back follows on stream_h)
@@ -250,23 +227,19 @@ struct vbx_ctx {
     cudaStream_t stream = nullptr;
     uint64_t* pkeys1 = nullptr;
     uint32_t* pvals[2] = {nullptr, nullptr};
-    vbx::SortPlan* sort_plan0 = nullptr;
+    vbx::SortPlan* sort_plan0 = nullptr;  // the point-key sort (vbx_sort.cuh)
     uint32_t* sort_status0 = nullptr;
     uint32_t* scan_status = nullptr;
-    uint32_t* big_list = nullptr;
-    uint32_t* first_bits = nullptr;
-    vbx::OrderScratch order_scratch{};
-    cudaStream_t side = nullptr;
+    uint32_t* big_list = nullptr;      // [max_points / 256 + 1] ids of the big bundles
+    uint32_t* first_bits = nullptr;    // [2][max_points / 32 + 1] first-occurrence bitmaps
+    vbx::OrderScratch order_scratch{};  // k_bundle_order's global tables
+    cudaStream_t side = nullptr;       // k_bundle_order runs here, beside k_merge
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   } lane[kLanes];
   bool async_ready = false;
   int prio_lo = 0, prio_hi = 0;  // stream priority range of the device
   cudaStream_t stream_e = nullptr;      // ray walk + block creation + record sort of asynchronously submitted scans
   cudaStream_t stream_s[kSortStreams] = {nullptr, nullptr};  // record sorts (set-private buffers: independent across scans)
-  cudaStream_t sort_stream = nullptr;   // non-null while an asynchronous back half is enqueued: the record sort goes here
-  cudaEvent_t walked_event = nullptr;   // ... after this event
-  cudaStream_t apply_stream = nullptr;  // ... and the apply kernels here
-  cudaEvent_t sorted_event = nullptr;   // ... after this event
   uint64_t async_seq = 0;
   uint32_t* d_hold = nullptr;           // device flag: a queued scan must be redone, later scans skip their back half
   uint64_t async_redone = 0;            // scans redone synchronously since vbx_create (reporting)
@@ -349,12 +322,8 @@ int mesh_download(vbx_ctx* c, int32_t* idx3, uint64_t* first_vertex, float* vert
 int esdf_add_robot_position(vbx_ctx* c, const float p[3]);
 int esdf_clear_state(vbx_ctx* c);
 int ensure_async(vbx_ctx* c);          // allocate the extra hand-off sets / front lanes
-void select_set(vbx_ctx* c, int k);     // point the context's scratch fields at hand-off set k / front lane l
-void select_lane(vbx_ctx* c, int l);
 int drain_async(vbx_ctx* c);           // wait for every asynchronously submitted scan, collect its results
 int set_n_blocks(vbx_ctx* c, uint32_t n);
-int alloc_order_scratch(vbx_ctx* c, vbx::OrderScratch* g, uint32_t** big_list, uint32_t** first_bits);
-void free_order_scratch(vbx::OrderScratch* g, uint32_t* big_list, uint32_t* first_bits);
 int init_bundle_order(vbx_ctx* c);     // rehash schedule + shared-memory opt-in of k_bundle_order
 int rebuild_hash(vbx_ctx* c);          // block hash rebuilt from slot_key (after removals / a pool overflow)
 void harvest_async(vbx_ctx* c, vbx_ctx::ScratchSet& S);  // collect a finished asynchronous scan's results

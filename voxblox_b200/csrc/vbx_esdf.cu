@@ -724,9 +724,9 @@ int esdf_create(vbx_ctx* c, const vbx_esdf_config* cfg) {
   const size_t nvox = (size_t)c->tab.max_blocks * c->vox_per_block;
   VBX_CUDA(c, cudaMalloc(reinterpret_cast<void**>(&c->tab.esdf), nvox * sizeof(EsdfVoxel)));
   // new Block<EsdfVoxel>: distance 0, all flags false, parent 0 (core/voxel.h:18-37)
-  VBX_CUDA(c, cudaMemsetAsync(c->tab.esdf, 0, nvox * sizeof(EsdfVoxel), c->stream));
-  VBX_CUDA(c, cudaMemsetAsync(c->tab.slot_has_esdf, 0, c->tab.max_blocks, c->stream));
-  VBX_CUDA(c, cudaMemsetAsync(c->tab.slot_esdf_updated, 0, c->tab.max_blocks, c->stream));
+  VBX_CUDA(c, cudaMemsetAsync(c->tab.esdf, 0, nvox * sizeof(EsdfVoxel), c->stream_main));
+  VBX_CUDA(c, cudaMemsetAsync(c->tab.slot_has_esdf, 0, c->tab.max_blocks, c->stream_main));
+  VBX_CUDA(c, cudaMemsetAsync(c->tab.slot_esdf_updated, 0, c->tab.max_blocks, c->stream_main));
   c->frontier_cap = std::min<uint64_t>(nvox, 1ull << 25);
   for (int i = 0; i < 2; ++i) {
     VBX_CUDA(c, cudaMalloc(reinterpret_cast<void**>(&c->frontier[i]), c->frontier_cap * sizeof(uint32_t)));
@@ -750,7 +750,7 @@ int esdf_create(vbx_ctx* c, const vbx_esdf_config* cfg) {
   c->esdf_ctas_wide = std::max(1, std::min(std::min(per_sm_r, per_sm_l), 4));
   c->esdf_grid_raise = sms;
   c->esdf_grid_lower = sms;
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   c->has_esdf = true;
   return VBX_OK;
 }
@@ -763,17 +763,18 @@ int esdf_clear_state(vbx_ctx* c) {
   c->esdf_pending_raise = c->esdf_pending_open = 0;
   if (c->n_blocks == 0) return VBX_OK;
   std::vector<uint8_t> eu(c->n_blocks);
-  VBX_CUDA(c, cudaMemcpyAsync(eu.data(), c->tab.slot_esdf_updated, c->n_blocks, cudaMemcpyDeviceToHost, c->stream));
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaMemcpyAsync(eu.data(), c->tab.slot_esdf_updated, c->n_blocks, cudaMemcpyDeviceToHost, c->stream_main));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   for (uint8_t& u : eu) u &= (uint8_t)~kEsdfPending;
-  VBX_CUDA(c, cudaMemcpyAsync(c->tab.slot_esdf_updated, eu.data(), c->n_blocks, cudaMemcpyHostToDevice, c->stream));
-  VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  VBX_CUDA(c, cudaMemcpyAsync(c->tab.slot_esdf_updated, eu.data(), c->n_blocks, cudaMemcpyHostToDevice, c->stream_main));
+  VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   return VBX_OK;
 }
 
 // EsdfIntegrator::addNewRobotPosition(position), esdf_integrator.cc:25-92
 int esdf_add_robot_position(vbx_ctx* c, const float p[3]) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
+  ScanState* st = c->set[0].d_state;  // the status block of hand-off set 0
   const vbx_esdf_config& cfg = c->ecfg;
   std::memset(c->esdf_counters, 0, sizeof(c->esdf_counters));
   uint64_t launches = 0;
@@ -799,29 +800,29 @@ int esdf_add_robot_position(vbx_ctx* c, const float p[3]) {
   // the per-axis lists ride in the seed-value scratch (floats; frontier_cap >> 1300 entries)
   float* d_xs[2] = {c->esdf_seed_val, c->esdf_seed_val + xs[0].size()};
   VBX_CUDA(c, cudaEventRecord(c->ev0, s));
-  VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
-  k_esdf_set_pending<<<1, 1, 0, s>>>(c->d_state, c->esdf_pending_raise, c->esdf_pending_open);
+  VBX_CUDA(c, cudaMemsetAsync(st, 0, sizeof(ScanState), s));
+  k_esdf_set_pending<<<1, 1, 0, s>>>(st, c->esdf_pending_raise, c->esdf_pending_open);
   for (int k = 0; k < 2; ++k) {
     if (S[k].n == 0) continue;
     VBX_CUDA(c, cudaMemcpyAsync(d_xs[k], xs[k].data(), xs[k].size() * sizeof(float), cudaMemcpyHostToDevice, s));
     const uint64_t n3 = (uint64_t)S[k].n * S[k].n * S[k].n;
-    k_esdf_sphere_blocks<<<grid_for(n3, 256), 256, 0, s>>>(S[k], c->tab, d_xs[k], c->d_state);
+    k_esdf_sphere_blocks<<<grid_for(n3, 256), 256, 0, s>>>(S[k], c->tab, d_xs[k], st);
     launches += 1;
   }
-  k_esdf_sphere_assign<<<grid_for(c->tab.max_blocks, 256), 256, 0, s>>>(c->tab, c->n_blocks, c->d_state);
+  k_esdf_sphere_assign<<<grid_for(c->tab.max_blocks, 256), 256, 0, s>>>(c->tab, c->n_blocks, st);
   launches += 2;
   for (int k = 0; k < 2; ++k) {
     if (S[k].n == 0) continue;
     const uint64_t n3 = (uint64_t)S[k].n * S[k].n * S[k].n;
-    k_esdf_sphere_apply<<<grid_for(n3, 256), 256, 0, s>>>(S[k], c->tab, d_xs[k], c->raise_q[0], c->frontier[0], c->d_state);
+    k_esdf_sphere_apply<<<grid_for(n3, 256), 256, 0, s>>>(S[k], c->tab, d_xs[k], c->raise_q[0], c->frontier[0], st);
     launches += 1;
   }
   VBX_CUDA(c, cudaEventRecord(c->ev1, s));
-  VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(c->set[0].h_state, st, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));  // (also keeps xs[] alive until the copies are done)
   VBX_CUDA(c, cudaGetLastError());
   VBX_CUDA(c, cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1));
-  const ScanState& h = *c->h_state;
+  const ScanState& h = *c->set[0].h_state;
   if (h.error & (kErrPoolFull | kErrHashFull)) return fail(c, VBX_E_CAPACITY, "block pool / hash full in addNewRobotPosition");
   if (h.error & kErrCoordRange) return fail(c, VBX_E_INVALID, "robot position sphere outside the +-2^20 block range");
   if (h.error & kErrUpdatesFull) return fail(c, VBX_E_CAPACITY, "ESDF wavefront queue capacity exceeded");
@@ -851,8 +852,8 @@ int esdf_update_blocks(vbx_ctx* c, const int32_t* idx3, uint64_t m, int incremen
   slots.reserve(m);
   std::vector<uint8_t> seen(c->n_blocks, 0), upd(c->n_blocks, 0);
   if (c->maybe_esdf_only && c->n_blocks) {
-    VBX_CUDA(c, cudaMemcpyAsync(upd.data(), c->tab.slot_updated, c->n_blocks, cudaMemcpyDeviceToHost, c->stream));
-    VBX_CUDA(c, cudaStreamSynchronize(c->stream));
+    VBX_CUDA(c, cudaMemcpyAsync(upd.data(), c->tab.slot_updated, c->n_blocks, cudaMemcpyDeviceToHost, c->stream_main));
+    VBX_CUDA(c, cudaStreamSynchronize(c->stream_main));
   }
   for (uint64_t i = 0; i < m; ++i) {
     auto it = c->host_key2slot.find(pack3(idx3[3 * i], idx3[3 * i + 1], idx3[3 * i + 2]));
@@ -865,7 +866,9 @@ int esdf_update_blocks(vbx_ctx* c, const int32_t* idx3, uint64_t m, int incremen
 
 static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_flag, const uint32_t* listed_slots,
                     uint32_t n_listed) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
+  ScanState* st = c->set[0].d_state;  // the status block of hand-off set 0
+  const ScanState& h = *c->set[0].h_state;
   std::memset(c->esdf_counters, 0, sizeof(c->esdf_counters));
   const vbx_esdf_config& cfg = c->ecfg;
   EsdfParams E;
@@ -891,7 +894,7 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
   uint64_t launches = 0;
   VBX_CUDA(c, cudaEventRecord(c->ev0, s));
   if (c->profiling) cudaEventRecord(c->sev[0], s);
-  VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
+  VBX_CUDA(c, cudaMemsetAsync(st, 0, sizeof(ScanState), s));
   if (c->n_blocks == 0) {
     VBX_CUDA(c, cudaStreamSynchronize(s));
     return VBX_OK;
@@ -905,7 +908,7 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
   // head of raise_q[0] / frontier[0]; this call's own entries are appended behind them)
   const bool pending = c->esdf_pending_raise || c->esdf_pending_open;
   if (pending) {
-    k_esdf_set_pending<<<1, 1, 0, s>>>(c->d_state, c->esdf_pending_raise, c->esdf_pending_open);
+    k_esdf_set_pending<<<1, 1, 0, s>>>(st, c->esdf_pending_raise, c->esdf_pending_open);
     launches += 1;
   }
   c->esdf_pending_raise = c->esdf_pending_open = 0;
@@ -921,7 +924,7 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
     nb = n_listed;
     if (nb > 0) {
       VBX_CUDA(c, cudaMemcpyAsync(c->esdf_block_list, listed_slots, (size_t)nb * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-      VBX_CUDA(c, cudaMemcpyAsync(&c->d_state->esdf_counts[0], &nb, sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+      VBX_CUDA(c, cudaMemcpyAsync(&st->esdf_counts[0], &nb, sizeof(uint32_t), cudaMemcpyHostToDevice, s));
       k_esdf_mark_listed<<<grid_for(nb, 256), 256, 0, s>>>(c->tab, c->esdf_block_list, nb);
       VBX_CUDA(c, cudaStreamSynchronize(s));  // the two host sources above are stack / vector memory
     }
@@ -929,7 +932,7 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
     // the list and its length (esdf_counts[0]) stay on the device: no host round trip in the middle of
     // the call; the launches below are sized for the upper bound (every slot) and the kernels stop at
     // the real count
-    k_esdf_block_list<<<grid_for(c->n_blocks, 256), 256, 0, s>>>(c->tab, c->n_blocks, batch, c->esdf_block_list, c->d_state);
+    k_esdf_block_list<<<grid_for(c->n_blocks, 256), 256, 0, s>>>(c->tab, c->n_blocks, batch, c->esdf_block_list, st);
     nb = c->n_blocks;
   }
   launches += 1;
@@ -938,13 +941,13 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
       // one thread block per voxel block, both slabs staged by the TMA
       const size_t slab_bytes = (size_t)c->vox_per_block * (sizeof(TsdfVoxel) + sizeof(EsdfVoxel));
       k_esdf_propagate<<<nb, (unsigned int)std::max<uint32_t>(32u, std::min<uint32_t>(1024u, c->vox_per_block)), slab_bytes, s>>>(
-          E, c->tab, c->esdf_block_list, nb, c->frontier[0], c->raise_q[0], c->esdf_seed_list, c->d_state);
+          E, c->tab, c->esdf_block_list, nb, c->frontier[0], c->raise_q[0], c->esdf_seed_list, st);
       launches += 1;
     }
     if (nb > 0 && incremental) {
       const unsigned int g = 148 * 8;
-      k_esdf_seed<<<g, 256, 0, s>>>(E, c->tab, c->esdf_seed_list, c->frontier[0], c->esdf_seed_val, c->d_state);
-      k_esdf_seed_commit<<<g, 256, 0, s>>>(E, c->tab, c->esdf_seed_list, c->esdf_seed_val, c->d_state);
+      k_esdf_seed<<<g, 256, 0, s>>>(E, c->tab, c->esdf_seed_list, c->frontier[0], c->esdf_seed_val, st);
+      k_esdf_seed_commit<<<g, 256, 0, s>>>(E, c->tab, c->esdf_seed_list, c->esdf_seed_val, st);
       launches += 2;
     }
     if (c->profiling) cudaEventRecord(c->sev[1], s);
@@ -954,24 +957,24 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
       c->esdf_grid_raise = c->esdf_grid_lower = c->esdf_sms * per_sm;
     }
     {
-      void* args[] = {&E, &c->tab, &c->raise_q[0], &c->raise_q[1], &c->frontier[0], &c->d_state};
+      void* args[] = {&E, &c->tab, &c->raise_q[0], &c->raise_q[1], &c->frontier[0], &st};
       VBX_CUDA(c, cudaLaunchCooperativeKernel((void*)k_esdf_raise, dim3(c->esdf_grid_raise), dim3(256), args, 0, s));
     }
     if (c->profiling) cudaEventRecord(c->sev[2], s);
     {
-      void* args[] = {&E, &c->tab, &c->frontier[0], &c->frontier[1], &c->esdf_touched, &c->d_state};
+      void* args[] = {&E, &c->tab, &c->frontier[0], &c->frontier[1], &c->esdf_touched, &st};
       VBX_CUDA(c, cudaLaunchCooperativeKernel((void*)k_esdf_lower, dim3(c->esdf_grid_lower), dim3(256), args, 0, s));
     }
-    k_esdf_parents<<<148 * 8, 256, 0, s>>>(E, c->tab, c->esdf_touched, c->d_state);
+    k_esdf_parents<<<148 * 8, 256, 0, s>>>(E, c->tab, c->esdf_touched, st);
     if (c->profiling) cudaEventRecord(c->sev[3], s);
     launches += 3;
     if (nb > 0 && !batch && clear_updated_flag) {
-      k_esdf_clear_tsdf_flag<<<grid_for(nb, 256), 256, 0, s>>>(c->tab, c->esdf_block_list, c->d_state);
+      k_esdf_clear_tsdf_flag<<<grid_for(nb, 256), 256, 0, s>>>(c->tab, c->esdf_block_list, st);
       launches += 1;
     }
   }
   VBX_CUDA(c, cudaEventRecord(c->ev1, s));
-  VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(c->set[0].h_state, st, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
   VBX_CUDA(c, cudaGetLastError());
   VBX_CUDA(c, cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1));
@@ -984,8 +987,8 @@ static int esdf_run(vbx_ctx* c, int batch, int incremental, int clear_updated_fl
       }
     }
   }
-  if (c->h_state->error & kErrUpdatesFull) return fail(c, VBX_E_CAPACITY, "ESDF wavefront queue capacity exceeded");
-  for (int i = 0; i < 7; ++i) c->esdf_counters[i] = c->h_state->esdf_counts[i];
+  if (h.error & kErrUpdatesFull) return fail(c, VBX_E_CAPACITY, "ESDF wavefront queue capacity exceeded");
+  for (int i = 0; i < 7; ++i) c->esdf_counters[i] = h.esdf_counts[i];
   c->esdf_counters[7] = launches;
   c->launches += launches;
   return VBX_OK;

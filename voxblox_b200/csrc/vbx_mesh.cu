@@ -306,7 +306,7 @@ void mesh_destroy(vbx_ctx* c) { mesh_free(c); }
 // MeshIntegrator::generateMesh(only_mesh_updated_blocks, clear_updated_flag), mesh_integrator.h:132-160
 int mesh_generate(vbx_ctx* c, const vbx_mesh_config* cfg, int only_updated, int clear_flag, uint64_t* n_blocks_out,
                   uint64_t* n_vertices_out) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   c->mesh_idx.clear();
   c->mesh_first_host.assign(1, 0);
   c->mesh_use_color = cfg->use_color != 0;
@@ -429,7 +429,7 @@ int mesh_generate(vbx_ctx* c, const vbx_mesh_config* cfg, int only_updated, int 
 
 // the result of the last mesh_generate, block by block in index order
 int mesh_download(vbx_ctx* c, int32_t* idx3, uint64_t* first_vertex, float* vertices, float* normals, uint8_t* colors) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
   const size_t nb = c->mesh_idx.size() / 3;
   if (idx3 && nb) std::memcpy(idx3, c->mesh_idx.data(), nb * 3 * sizeof(int32_t));
   if (first_vertex) std::memcpy(first_vertex, c->mesh_first_host.data(), c->mesh_first_host.size() * sizeof(uint64_t));

@@ -1909,12 +1909,12 @@ int init_bundle_order(vbx_ctx* c) {
 
 static inline unsigned int grid_for(uint64_t n, int block) { return (unsigned int)((n + block - 1) / block); }
 
-static int check_state_errors(vbx_ctx* c, uint32_t err) {
-  err &= kFatalErrors;
+static int check_state_errors(vbx_ctx* c, const ScanState& h) {
+  const uint32_t err = h.error & kFatalErrors;
   if (!err) return VBX_OK;
   if (err & kErrPoolFull) {
     // the surplus hash entries of this call have no pool slot: drop them, or later calls would find them
-    if (c->h_state->n_blocks) c->n_blocks = c->h_state->n_blocks;
+    if (h.n_blocks) c->n_blocks = h.n_blocks;
     rebuild_hash(c);
   }
   std::string m = "device reported:";
@@ -1929,13 +1929,14 @@ namespace {
 struct Marks {
   vbx_ctx* c;
   cudaStream_t s;
+  bool on;  // stage profiling (vbx_set_stage_profiling); pipelined scans run without: the events would serialise the streams
   int n = 0;
   int stage[20];
   void begin() {
-    if (c->profiling) cudaEventRecord(c->sev[0], s);
+    if (on) cudaEventRecord(c->sev[0], s);
   }
   void mark(int stage_just_finished) {
-    if (c->profiling && n < 19) {
+    if (on && n < 19) {
       cudaEventRecord(c->sev[n + 1], s);
       stage[n++] = stage_just_finished;
     }
@@ -1950,20 +1951,32 @@ struct Marks {
     }
   }
 };
+
+// Where the back half of a scan runs: the ray walk and block creation on `walk`, the record sort on `sort`,
+// the apply kernels on `apply`.  A stage on another stream than the one before it waits for the hand-off
+// event (`walked`, `sorted`); synchronous calls run all three on the main stream without hand-off events.
+struct Stages {
+  cudaStream_t walk, sort, apply;
+  cudaEvent_t walked, sorted;
+};
+
+// the map's tables as one scan's kernels see them: with the hand-off set's own touched-block list
+Tables scan_tables(const vbx_ctx* c, const vbx_ctx::ScratchSet& S) {
+  Tables t = c->tab;
+  t.touched_list = S.touched_list;
+  return t;
+}
 }  // namespace
 
-// The engine's own stable radix sort (vbx_sort.cuh): one launch.  n lives on the device (d_n) or is n_fixed;
-// n_hint sizes the grid (tiles are handed out by ticket, so any grid sorts any n).  result_in_a: the sorted
-// pairs end in buffer A whatever the number of passes (otherwise SortPlan::final_buf says where they are).
+// The engine's own stable radix sort (vbx_sort.cuh): one launch on stream s.  n lives on the device (d_n) or
+// is n_fixed; n_hint sizes the grid (tiles are handed out by ticket, so any grid sorts any n).  result_in_a: the
+// sorted pairs end in buffer A whatever the number of passes (otherwise SortPlan::final_buf says where they are).
 template <typename KeyT>
-static int own_sort(vbx_ctx* c, int which, KeyT* keys_a, uint32_t* vals_a, KeyT* keys_b, uint32_t* vals_b,
-                    const unsigned long long* d_n, uint32_t n_fixed, uint64_t n_hint, int key_bits, bool result_in_a,
-                    uint64_t* launches, const uint32_t* d_key_bits = nullptr, bool plan_cleared = false) {
-  cudaStream_t s = c->stream;
+static int own_sort(vbx_ctx* c, cudaStream_t s, SortPlan* plan, uint32_t* status, uint32_t tiles_cap, KeyT* keys_a,
+                    uint32_t* vals_a, KeyT* keys_b, uint32_t* vals_b, const unsigned long long* d_n, uint32_t n_fixed,
+                    uint64_t n_hint, int key_bits, bool result_in_a, uint64_t* launches,
+                    const uint32_t* d_key_bits = nullptr, bool plan_cleared = false) {
   const int passes = std::min(kMaxPasses, (key_bits + 7) / 8);
-  SortPlan* plan = c->sort_plan[which];
-  uint32_t* status = c->sort_status[which];
-  const uint32_t tiles_cap = c->sort_tiles_cap[which];
   if (!plan_cleared) VBX_CUDA(c, cudaMemsetAsync(plan, 0, sizeof(SortPlan), s));  // (else: an earlier kernel of the stream did)
   const uint64_t tiles_hint = std::max<uint64_t>(1, (n_hint + kSortTile - 1) / kSortTile);
   const unsigned int grid = (unsigned int)std::min<uint64_t>(std::min<uint64_t>(tiles_cap, tiles_hint), (uint64_t)c->grid_sms * 2);
@@ -1980,10 +1993,11 @@ constexpr int kOrderGrid = 32;  // blocks of the cooperative k_bundle_order laun
 // -- every SM busy with other scans' kernels -- it waits for one to drain.  A scan with more bundles than the
 // request covers is still ordered correctly: the kernel falls back to its global-memory stages.
 template <typename KeyT>
-static int launch_bundle_order(vbx_ctx* c, cudaStream_t so, const ScanParams& P, const KeyT* keys, const uint32_t* vals) {
-  k_order_prefix<<<1, kOrderThreads, 0, so>>>(P.n, c->first_bits, c->order_scratch, c->d_state);
+static int launch_bundle_order(vbx_ctx* c, vbx_ctx::ScratchSet& S, vbx_ctx::FrontLane& F, cudaStream_t so,
+                               const ScanParams& P, const KeyT* keys, const uint32_t* vals) {
+  k_order_prefix<<<1, kOrderThreads, 0, so>>>(P.n, F.first_bits, F.order_scratch, S.d_state);
   k_order_heads<KeyT><<<std::min<unsigned int>(grid_for(P.n, 256), 148 * 2), 256, 0, so>>>(
-      P, keys, vals, c->order_inv, c->head_list, c->first_bits, c->order_scratch, c->d_state);
+      P, keys, vals, c->order_inv, S.head_list, F.first_bits, F.order_scratch, S.d_state);
   RehashSchedule rs = c->rehash;
   size_t smem_bytes = c->order_smem_bytes;
   unsigned int grid = kOrderGrid;
@@ -1998,11 +2012,11 @@ static int launch_bundle_order(vbx_ctx* c, cudaStream_t so, const ScanParams& P,
       grid = 1;  // the single-block form; block 0 is the only one that would work
     }
   }
-  OrderScratch g = c->order_scratch;
+  OrderScratch g = F.order_scratch;
   uint32_t smem_words = (uint32_t)(smem_bytes / 4);
-  uint32_t* ray_list = c->ray_list;
-  uint32_t* cta_tot = c->order_scratch.cta_tot;
-  ScanState* st = c->d_state;
+  uint32_t* ray_list = S.ray_list;
+  uint32_t* cta_tot = F.order_scratch.cta_tot;
+  ScanState* st = S.d_state;
   void* args[] = {&rs, &g, &smem_words, &ray_list, &cta_tot, &st};
   if (grid == 1) {
     // an ordinary launch: nothing about it has to be co-scheduled
@@ -2015,63 +2029,65 @@ static int launch_bundle_order(vbx_ctx* c, cudaStream_t so, const ScanParams& P,
 
 // Stages up to and including k_assign: everything that decides WHICH voxels are updated.
 template <typename KeyT>
-static int front_half(vbx_ctx* c, ScanParams& P, const float* d_xyz, const uint8_t* d_rgba, const uint32_t* order,
-                      Marks& mk, uint64_t* launches, const KeyT** keys_out) {
-  cudaStream_t s = c->stream;
+static int front_half(vbx_ctx* c, vbx_ctx::ScratchSet& S, vbx_ctx::FrontLane& F, cudaStream_t s, ScanParams& P,
+                      const float* d_xyz, const uint8_t* d_rgba, const uint32_t* order, Marks& mk, uint64_t* launches,
+                      const KeyT** keys_out) {
   const uint32_t n = P.n;
   const int TB = 256;
+  const Tables tab = scan_tables(c, S);
   const KeyT* keys = nullptr;
   const uint32_t* vals = nullptr;
   const uint32_t* scan_perm = nullptr;
   const uint32_t* scan_limit = nullptr;
   if (P.kind == VBX_MERGED) {
-    KeyT* k0 = reinterpret_cast<KeyT*>(c->pkeys[0]);
-    KeyT* k1 = reinterpret_cast<KeyT*>(c->pkeys[1]);
+    KeyT* k0 = reinterpret_cast<KeyT*>(S.pkeys0);
+    KeyT* k1 = reinterpret_cast<KeyT*>(F.pkeys1);
     k_point_bounds<<<std::min<unsigned int>(grid_for(n, TB), 148 * 4), TB, 0, s>>>(
-        P, d_xyz, c->first_bits, c->sort_plan[0], c->scan_status, (n + 1 + kScanTile - 1) / kScanTile + 1, c->d_state);
-    k_point_keys<KeyT><<<grid_for(n, TB), TB, 0, s>>>(P, d_xyz, order, k0, c->pvals[0], c->d_state);
+        P, d_xyz, F.first_bits, F.sort_plan0, F.scan_status, (n + 1 + kScanTile - 1) / kScanTile + 1, S.d_state);
+    k_point_keys<KeyT><<<grid_for(n, TB), TB, 0, s>>>(P, d_xyz, order, k0, F.pvals[0], S.d_state);
     mk.mark(0);
     // the bits in use are known on the device only (ScanState::key_bits): passes beyond them exit at once
-    if (int rc = own_sort<KeyT>(c, 0, k0, c->pvals[0], k1, c->pvals[1], nullptr, n, n, 8 * (int)sizeof(KeyT), true, launches,
-                                &c->d_state->key_bits, /*plan_cleared=*/true)) {
+    if (int rc = own_sort<KeyT>(c, s, F.sort_plan0, F.sort_status0, c->sort_tiles_cap[0], k0, F.pvals[0], k1, F.pvals[1],
+                                nullptr, n, n, 8 * (int)sizeof(KeyT), true, launches, &S.d_state->key_bits,
+                                /*plan_cleared=*/true)) {
       return rc;
     }
     keys = k0;
-    vals = c->pvals[0];
+    vals = F.pvals[0];
     mk.mark(1);
-    k_heads<KeyT><<<grid_for((uint64_t)n + 1, TB), TB, 0, s>>>(P, keys, vals, c->order_inv, c->head_list, c->big_list,
-                                                               c->first_bits, c->cnt, c->d_state);
+    k_heads<KeyT><<<grid_for((uint64_t)n + 1, TB), TB, 0, s>>>(P, keys, vals, c->order_inv, S.head_list, F.big_list,
+                                                               F.first_bits, S.cnt, S.d_state);
     // The reference's bundle order (ray_list[rank] = bundle id, vbx_order.cuh) is one thread block's work
     // and the fold (k_merge) does not need it: the two run side by side.  (With stage profiling on they
     // run one after the other so that each gets its own time.)
-    cudaStream_t so = c->profiling ? s : c->side_stream;
+    cudaStream_t so = mk.on ? s : F.side;
     if (so != s) {
-      VBX_CUDA(c, cudaEventRecord(c->ev_fork, s));
-      VBX_CUDA(c, cudaStreamWaitEvent(so, c->ev_fork, 0));
+      VBX_CUDA(c, cudaEventRecord(F.ev_fork, s));
+      VBX_CUDA(c, cudaStreamWaitEvent(so, F.ev_fork, 0));
     }
-    if (int rc = launch_bundle_order<KeyT>(c, so, P, keys, vals)) return rc;
-    if (so != s) VBX_CUDA(c, cudaEventRecord(c->ev_join, so));
+    if (int rc = launch_bundle_order<KeyT>(c, S, F, so, P, keys, vals)) return rc;
+    if (so != s) VBX_CUDA(c, cudaEventRecord(F.ev_join, so));
     mk.mark(12);
-    k_merge<KeyT><<<c->grid_sms * 4, 192, 0, s>>>(P, d_xyz, d_rgba, keys, vals, c->head_list, c->big_list, c->ray_p, c->ray_a,
-                                           c->ray_c, c->cnt, c->d_state);
+    k_merge<KeyT><<<c->grid_sms * 4, 192, 0, s>>>(P, d_xyz, d_rgba, keys, vals, S.head_list, F.big_list, S.ray_p, S.ray_a,
+                                           S.ray_c, S.cnt, S.d_state);
     mk.mark(8);
     *launches += 8;
     if (!P.single_walk) {
       // the bundle count is only known on the device: launch for the worst case (every
       // point its own bundle); surplus threads exit on the first load
-      k_rays_count<KeyT><<<grid_for(n, 128), 128, 0, s>>>(P, c->tab, d_xyz, d_rgba, order, keys, c->head_list,
-                                                           c->ray_p, c->ray_a, c->ray_c, c->cnt, c->set_start,
-                                                           c->set_observed, c->d_state);
+      k_rays_count<KeyT><<<grid_for(n, 128), 128, 0, s>>>(P, tab, d_xyz, d_rgba, order, keys, S.head_list,
+                                                           S.ray_p, S.ray_a, S.ray_c, S.cnt, c->set_start,
+                                                           c->set_observed, S.d_state);
       *launches += 1;
     }
-    if (so != s) VBX_CUDA(c, cudaStreamWaitEvent(s, c->ev_join, 0));
+    if (so != s) VBX_CUDA(c, cudaStreamWaitEvent(s, F.ev_join, 0));
     // record offsets in RANK order: off[rank] = sum of cnt[ray_list[r]] over r < rank
-    scan_perm = c->ray_list;
-    scan_limit = &c->d_state->n_ray_list;
+    scan_perm = S.ray_list;
+    scan_limit = &S.d_state->n_ray_list;
   } else {
-    k_rays_count<KeyT><<<grid_for((uint64_t)n + 1, 128), 128, 0, s>>>(P, c->tab, d_xyz, d_rgba, order, keys,
-                                                                       c->head_list, c->ray_p, c->ray_a, c->ray_c, c->cnt,
-                                                                       c->set_start, c->set_observed, c->d_state);
+    k_rays_count<KeyT><<<grid_for((uint64_t)n + 1, 128), 128, 0, s>>>(P, tab, d_xyz, d_rgba, order, keys,
+                                                                       S.head_list, S.ray_p, S.ray_a, S.ray_c, S.cnt,
+                                                                       c->set_start, c->set_observed, S.d_state);
     *launches += 1;
   }
   mk.mark(2);
@@ -2079,10 +2095,10 @@ static int front_half(vbx_ctx* c, ScanParams& P, const float* d_xyz, const uint8
     // record offsets; the scan's last position also settles the call's update count (total_found, total_updates,
     // kErrUpdatesFull: too many for one pass; nothing downstream runs on a call that failed)
     const uint32_t tiles = (n + 1 + kScanTile - 1) / kScanTile;
-    if (P.kind != VBX_MERGED) VBX_CUDA(c, cudaMemsetAsync(c->scan_status, 0, (size_t)(tiles + 1) * sizeof(uint32_t), s));  // (Merged: k_point_bounds did)
+    if (P.kind != VBX_MERGED) VBX_CUDA(c, cudaMemsetAsync(F.scan_status, 0, (size_t)(tiles + 1) * sizeof(uint32_t), s));  // (Merged: k_point_bounds did)
     k_exclusive_scan<<<std::min<uint32_t>(tiles, 148 * 4), kSortThreads, 0, s>>>(
-        c->cnt, scan_perm, scan_limit, c->off, n + 1, c->scan_status + 1, c->scan_status, &c->d_state->total_found,
-        &c->d_state->total_updates, &c->d_state->error, (unsigned long long)c->max_updates, kErrUpdatesFull);
+        S.cnt, scan_perm, scan_limit, S.off, n + 1, F.scan_status + 1, F.scan_status, &S.d_state->total_found,
+        &S.d_state->total_updates, &S.d_state->error, (unsigned long long)c->max_updates, kErrUpdatesFull);
   }
   mk.mark(3);
   *launches += 1;
@@ -2091,43 +2107,41 @@ static int front_half(vbx_ctx* c, ScanParams& P, const float* d_xyz, const uint8
 }
 
 // update-record sort + the apply kernels
-static int sort_and_apply(vbx_ctx* c, const ScanParams& P, unsigned long long K, uint32_t n_touched, Marks& mk,
-                          uint64_t* launches) {
-  cudaStream_t s = c->stream;
+static int sort_and_apply(vbx_ctx* c, vbx_ctx::ScratchSet& S, const Stages& st, const ScanParams& P, unsigned long long K,
+                          uint32_t n_touched, Marks& mk, uint64_t* launches) {
   RecordView rv;
   {
     // K and the number of touched blocks are only known on the device: sort on every bit a
     // record key can have; passes whose digit is uniform are skipped on the device
     const int key_bits = 32;
-    if (c->sort_stream) {
+    if (st.walked) {
       // pipelined submission: the record sort works on buffers private to this scan, so it leaves
       // the walk stream (which the next scan's ray walk is waiting for)
-      VBX_CUDA(c, cudaEventRecord(c->walked_event, s));
-      VBX_CUDA(c, cudaStreamWaitEvent(c->sort_stream, c->walked_event, 0));
-      s = c->sort_stream;
-      c->stream = s;
+      VBX_CUDA(c, cudaEventRecord(st.walked, st.walk));
+      VBX_CUDA(c, cudaStreamWaitEvent(st.sort, st.walked, 0));
     }
-    if (int rc = own_sort<uint32_t>(c, 1, c->ckeys[0], c->cvals[0], c->ckeys[1], c->cvals[1], &c->d_state->total_updates,
-                                     0, c->record_hint, key_bits, false, launches, &c->d_state->rec_key_bits,
-                                     /*plan_cleared=*/true)) {
+    if (int rc = own_sort<uint32_t>(c, st.sort, S.sort_plan1, S.sort_status1, c->sort_tiles_cap[1], S.ckeys[0], S.cvals[0],
+                                     S.ckeys[1], S.cvals[1], &S.d_state->total_updates, 0, c->record_hint, key_bits, false,
+                                     launches, &S.d_state->rec_key_bits, /*plan_cleared=*/true)) {
       return rc;
     }
-    rv.keys[0] = c->ckeys[0];
-    rv.keys[1] = c->ckeys[1];
-    rv.vals[0] = c->cvals[0];
-    rv.vals[1] = c->cvals[1];
-    rv.plan = c->sort_plan[1];
-    rv.d_total = &c->d_state->total_updates;
+    rv.keys[0] = S.ckeys[0];
+    rv.keys[1] = S.ckeys[1];
+    rv.vals[0] = S.cvals[0];
+    rv.vals[1] = S.cvals[1];
+    rv.plan = S.sort_plan1;
+    rv.d_total = &S.d_state->total_updates;
     rv.total_fixed = 0;
   }
   mk.mark(6);
-  if (c->apply_stream) {
+  if (st.sorted) {
     // pipelined submission: the apply kernels run on their own stream behind the sort, so the
     // next scan's ray walk can start while this scan's voxels are still being written
-    VBX_CUDA(c, cudaEventRecord(c->sorted_event, s));
-    VBX_CUDA(c, cudaStreamWaitEvent(c->apply_stream, c->sorted_event, 0));
-    s = c->apply_stream;
+    VBX_CUDA(c, cudaEventRecord(st.sorted, st.sort));
+    VBX_CUDA(c, cudaStreamWaitEvent(st.apply, st.sorted, 0));
   }
+  cudaStream_t s = st.apply;
+  const Tables tab = scan_tables(c, S);
   const unsigned int g_short = c->grid_sms * 8;
   LongRuns lr;
   lr.start = c->long_list;
@@ -2137,47 +2151,49 @@ static int sort_and_apply(vbx_ctx* c, const ScanParams& P, unsigned long long K,
   lr.item_start = c->verify_start;
   lr.rec_sdf = c->rec_sdf;
   lr.rec_w = c->rec_w;
-  k_apply_short<<<g_short, 256, 0, s>>>(P, c->tab, rv, c->ray_a, c->ray_c, lr, c->d_state);
-  k_apply_verify<<<c->grid_sms * 8, 128, 0, s>>>(P, c->tab, rv, c->ray_a, c->ray_c, lr, c->d_state);
-  k_apply_long<<<c->grid_sms * 4, 128, 0, s>>>(P, c->tab, rv, c->ray_a, c->ray_c, lr, c->d_state);
+  k_apply_short<<<g_short, 256, 0, s>>>(P, tab, rv, S.ray_a, S.ray_c, lr, S.d_state);
+  k_apply_verify<<<c->grid_sms * 8, 128, 0, s>>>(P, tab, rv, S.ray_a, S.ray_c, lr, S.d_state);
+  k_apply_long<<<c->grid_sms * 4, 128, 0, s>>>(P, tab, rv, S.ray_a, S.ray_c, lr, S.d_state);
   mk.mark(7);
   *launches += 3;
   return VBX_OK;
 }
 
 template <typename KeyT>
-static int back_half(vbx_ctx* c, const ScanParams& P, const KeyT* keys, unsigned long long K, uint32_t n_touched,
-                     Marks& mk, uint64_t* launches) {
-  cudaStream_t s = c->stream;
+static int back_half(vbx_ctx* c, vbx_ctx::ScratchSet& S, const Stages& st, const ScanParams& P, const KeyT* keys,
+                     unsigned long long K, uint32_t n_touched, Marks& mk, uint64_t* launches) {
+  cudaStream_t s = st.walk;
   const uint32_t n = P.n;
+  const Tables tab = scan_tables(c, S);
   if (P.kind == VBX_MERGED && P.single_walk) {
     // a few thousand bundles of 100-300 steps: one warp per ray
-    k_rays_emit_warp<KeyT><<<c->grid_sms * 8, 128, 0, s>>>(P, c->tab, keys, c->ray_list, c->head_list, c->ray_p, c->cnt, c->off,
-                                                   c->ckeys[0], c->cvals[0], c->d_state);
+    k_rays_emit_warp<KeyT><<<c->grid_sms * 8, 128, 0, s>>>(P, tab, keys, S.ray_list, S.head_list, S.ray_p, S.cnt, S.off,
+                                                   S.ckeys[0], S.cvals[0], S.d_state);
   } else {
-    k_rays_emit<KeyT><<<grid_for(n, 128), 128, 0, s>>>(P, c->tab, keys, c->ray_list, c->head_list, c->ray_p, c->cnt, c->off,
-                                                        c->ckeys[0], c->cvals[0], c->d_state);
+    k_rays_emit<KeyT><<<grid_for(n, 128), 128, 0, s>>>(P, tab, keys, S.ray_list, S.head_list, S.ray_p, S.cnt, S.off,
+                                                        S.ckeys[0], S.cvals[0], S.d_state);
   }
   mk.mark(5);
   k_assign<<<grid_for(std::max<uint32_t>(c->tab.max_blocks, 1024), 256), 256, 0, s>>>(
-      c->tab, c->d_nblocks + c->nb_cur, c->d_nblocks + (c->nb_cur ^ 1), c->sort_plan[1], c->d_state);
+      tab, c->d_nblocks + c->nb_cur, c->d_nblocks + (c->nb_cur ^ 1), S.sort_plan1, S.d_state);
   c->nb_cur ^= 1;
   mk.mark(4);
   *launches += 2;
-  return sort_and_apply(c, P, K, n_touched, mk, launches);
+  return sort_and_apply(c, S, st, P, K, n_touched, mk, launches);
 }
 
 // The back half of a call whose K exceeds max_updates_per_pass, in passes (see integrate_device).
 template <typename KeyT>
-static int apply_in_passes(vbx_ctx* c, ScanParams P, const KeyT* keys, Marks& mk, uint64_t* launches) {
-  cudaStream_t s = c->stream;
+static int apply_in_passes(vbx_ctx* c, vbx_ctx::ScratchSet& S, const Stages& st, ScanParams P, const KeyT* keys, Marks& mk,
+                           uint64_t* launches) {
+  cudaStream_t s = st.walk;
   const uint32_t n = P.n;
   std::vector<uint32_t> off(n + 1);
-  VBX_CUDA(c, cudaMemcpyAsync(off.data(), c->off, (size_t)(n + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(off.data(), S.off, (size_t)(n + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
   if (P.kind == VBX_MERGED) {
     // the scan wrote the offsets of the bundles and, at [n], the total; ranks past the last bundle hold nothing
-    const uint32_t nr = std::min(c->h_state->n_ray_list, n);
+    const uint32_t nr = std::min(S.h_state->n_ray_list, n);
     for (uint32_t i = nr + 1; i < n; ++i) off[i] = off[n];
   }
   uint32_t lo = 0, passes = 0;
@@ -2194,9 +2210,9 @@ static int apply_in_passes(vbx_ctx* c, ScanParams P, const KeyT* keys, Marks& mk
       P.emit_lo = lo;
       P.emit_hi = hi;
       P.emit_base = off[lo];
-      k_pass_begin<<<1, 1, 0, s>>>(c->d_state, kp);
+      k_pass_begin<<<1, 1, 0, s>>>(S.d_state, kp);
       *launches += 1;
-      if (int rc = back_half<KeyT>(c, P, keys, kp, 0, mk, launches)) return rc;
+      if (int rc = back_half<KeyT>(c, S, st, P, keys, kp, 0, mk, launches)) return rc;
       ++passes;
     }
     lo = hi;
@@ -2262,7 +2278,11 @@ int integrate_device(vbx_ctx* c, int kind, const float q[4], const float t[3], c
   if (kind < VBX_SIMPLE || kind > VBX_FAST) return fail(c, VBX_E_INVALID, "Unknown TSDF integrator type");
   if (n64 > c->max_points) return fail(c, VBX_E_CAPACITY, "cloud larger than max_points_per_scan");
   const uint32_t n = (uint32_t)n64;
-  cudaStream_t s = c->stream;
+  // synchronous calls work on hand-off set 0 and front lane 0, every stage on the main stream
+  vbx_ctx::ScratchSet& S = c->set[0];
+  vbx_ctx::FrontLane& F = c->lane[0];
+  cudaStream_t s = c->stream_main;
+  const Stages st{s, s, s, nullptr, nullptr};
   const vbx_tsdf_config& cfg = c->cfg;
   std::memset(c->counters, 0, sizeof(c->counters));
   uint64_t launches = 0;
@@ -2271,7 +2291,7 @@ int integrate_device(vbx_ctx* c, int kind, const float q[4], const float t[3], c
   fill_params(c, kind, q, t, n, freespace, P);
 
   VBX_CUDA(c, cudaEventRecord(c->ev0, s));
-  VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
+  VBX_CUDA(c, cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), s));
   if (n == 0) {
     VBX_CUDA(c, cudaEventRecord(c->ev1, s));
     VBX_CUDA(c, cudaStreamSynchronize(s));
@@ -2279,19 +2299,18 @@ int integrate_device(vbx_ctx* c, int kind, const float q[4], const float t[3], c
     return VBX_OK;
   }
   const int TB = 256;
-  Marks mk;
-  mk.c = c;
-  mk.s = s;
+  Marks mk{c, s, c->profiling};
   mk.begin();
 
   const uint32_t* order = nullptr;
   if (cfg.integration_order_mode == 1) {
     // SortedThreadSafeIndex: ascending |p|^2 (stable here; std::sort leaves ties unspecified)
-    k_sqnorm_keys<<<grid_for(n, TB), TB, 0, s>>>(n, d_xyz, c->pkeys[0], c->pvals[0]);
-    if (int rc = own_sort<uint64_t>(c, 0, c->pkeys[0], c->pvals[0], c->pkeys[1], c->pvals[1], nullptr, n, n, 64, true, &launches)) {
+    k_sqnorm_keys<<<grid_for(n, TB), TB, 0, s>>>(n, d_xyz, S.pkeys0, F.pvals[0]);
+    if (int rc = own_sort<uint64_t>(c, s, F.sort_plan0, F.sort_status0, c->sort_tiles_cap[0], S.pkeys0, F.pvals[0], F.pkeys1,
+                                    F.pvals[1], nullptr, n, n, 64, true, &launches)) {
       return rc;
     }
-    VBX_CUDA(c, cudaMemcpyAsync(c->order, c->pvals[0], n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+    VBX_CUDA(c, cudaMemcpyAsync(c->order, F.pvals[0], n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
     k_invert_order<<<grid_for(n, TB), TB, 0, s>>>(n, c->order, c->order_inv);
     order = c->order;
     launches += 2;
@@ -2302,51 +2321,51 @@ int integrate_device(vbx_ctx* c, int kind, const float q[4], const float t[3], c
   const uint64_t* keys64 = nullptr;
   unsigned long long K = 0;
   uint32_t n_touched = 0;
-  if (int rc = front_half<uint64_t>(c, P, d_xyz, d_rgba, order, mk, &launches, &keys64)) return rc;
+  if (int rc = front_half<uint64_t>(c, S, F, s, P, d_xyz, d_rgba, order, mk, &launches, &keys64)) return rc;
   {
     // own sort: K stays on the device, the whole call is enqueued without a host round trip
-    if (int rc = back_half<uint64_t>(c, P, keys64, 0, 0, mk, &launches)) return rc;
+    if (int rc = back_half<uint64_t>(c, S, st, P, keys64, 0, 0, mk, &launches)) return rc;
     VBX_CUDA(c, cudaEventRecord(c->ev1, s));
-    VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+    VBX_CUDA(c, cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
     VBX_CUDA(c, cudaStreamSynchronize(s));
-    if (c->h_state->error == kErrUpdatesFull) {
+    if (S.h_state->error == kErrUpdatesFull) {
       // More update records than one pass holds.  Nothing was emitted or applied; the per-ray
       // tables, counts and offsets of the front half stand.  Apply the call in passes over
       // contiguous ray-slot ranges: every voxel still sees its updates in ray-rank order, so
       // the result is the one-pass result bit for bit.
       chunk_blocks_before = c->n_blocks;
-      if (int rc = apply_in_passes<uint64_t>(c, P, keys64, mk, &launches)) return rc;
+      if (int rc = apply_in_passes<uint64_t>(c, S, st, P, keys64, mk, &launches)) return rc;
       chunked = true;
       VBX_CUDA(c, cudaEventRecord(c->ev1, s));
-      VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+      VBX_CUDA(c, cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
       VBX_CUDA(c, cudaStreamSynchronize(s));
     }
-    if (int rc = check_state_errors(c, c->h_state->error)) return rc;
-    c->n_blocks = c->h_state->n_blocks;
-    K = c->h_state->total_found;
-    n_touched = c->h_state->n_touched;
+    if (int rc = check_state_errors(c, *S.h_state)) return rc;
+    c->n_blocks = S.h_state->n_blocks;
+    K = S.h_state->total_found;
+    n_touched = S.h_state->n_touched;
   }
   VBX_CUDA(c, cudaEventRecord(c->ev1, s));
-  VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
   VBX_CUDA(c, cudaGetLastError());
   VBX_CUDA(c, cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1));
   mk.collect();
   c->launches += launches;
-  c->counters[0] = c->h_state->n_rays;
-  if (kind == VBX_MERGED) c->bundle_hint = std::max(c->h_state->n_rays, c->h_state->n_clear_rays);
-  c->counters[1] = c->h_state->n_clear_rays;
+  c->counters[0] = S.h_state->n_rays;
+  if (kind == VBX_MERGED) c->bundle_hint = std::max(S.h_state->n_rays, S.h_state->n_clear_rays);
+  c->counters[1] = S.h_state->n_clear_rays;
   c->counters[2] = K;
   if (K) c->record_hint = K;
-  c->counters[3] = c->h_state->n_voxels;
+  c->counters[3] = S.h_state->n_voxels;
   c->counters[4] = n_touched;
-  c->counters[5] = chunked ? (uint64_t)(c->n_blocks - chunk_blocks_before) : (uint64_t)c->h_state->n_new;
+  c->counters[5] = chunked ? (uint64_t)(c->n_blocks - chunk_blocks_before) : (uint64_t)S.h_state->n_new;
   c->counters[11] = chunked ? c->last_passes : 1;
-  c->counters[9] = c->h_state->n_refold;
-  c->counters[10] = c->h_state->refold_members;
-  c->counters[12] = c->h_state->key_bits;
-  c->counters[6] = (kind == VBX_MERGED) ? c->h_state->n_valid_points
-                                        : (uint64_t)c->h_state->n_rays + c->h_state->n_clear_rays;
+  c->counters[9] = S.h_state->n_refold;
+  c->counters[10] = S.h_state->refold_members;
+  c->counters[12] = S.h_state->key_bits;
+  c->counters[6] = (kind == VBX_MERGED) ? S.h_state->n_valid_points
+                                        : (uint64_t)S.h_state->n_rays + S.h_state->n_clear_rays;
   c->counters[7] = launches;
   return VBX_OK;
 }
@@ -2376,17 +2395,17 @@ int integrate_async(vbx_ctx* c, int kind, const float q[4], const float t[3], co
     const float* dx = xyz;
     const uint8_t* dr = rgba;
     if (!on_device && n64) {
-      VBX_CUDA(c, cudaMemcpyAsync(c->d_xyz, xyz, n64 * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-      VBX_CUDA(c, cudaMemcpyAsync(c->d_rgba, rgba, n64 * 4, cudaMemcpyHostToDevice, c->stream));
-      dx = c->d_xyz;
-      dr = c->d_rgba;
+      vbx_ctx::ScratchSet& S0 = c->set[0];
+      VBX_CUDA(c, cudaMemcpyAsync(S0.d_xyz, xyz, n64 * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream_main));
+      VBX_CUDA(c, cudaMemcpyAsync(S0.d_rgba, rgba, n64 * 4, cudaMemcpyHostToDevice, c->stream_main));
+      dx = S0.d_xyz;
+      dr = S0.d_rgba;
     }
     return integrate_device(c, kind, q, t, dx, dr, n64, freespace);
   }
   if (int rc = ensure_async(c)) return rc;
   const uint32_t n = (uint32_t)n64;
-  const int k = (int)(c->async_seq % c->sets_in_use);
-  vbx_ctx::ScratchSet& S = c->set[k];
+  vbx_ctx::ScratchSet& S = c->set[c->async_seq % c->sets_in_use];
   vbx_ctx::FrontLane& F = c->lane[c->async_seq % c->lanes_in_use];
   const auto t_enter = std::chrono::steady_clock::now();
   if (S.in_flight) {  // bounded run-ahead: wait for the scan that used this hand-off set
@@ -2398,21 +2417,11 @@ int integrate_async(vbx_ctx* c, int kind, const float q[4], const float t[3], co
       if (int rc = drain_async(c)) return rc;
     }
   }
-  select_set(c, k);
-  select_lane(c, (int)(c->async_seq % c->lanes_in_use));
   ScanParams P;
   fill_params(c, kind, q, t, n, freespace, P);
   uint64_t launches = 0;
-  Marks mk;
-  mk.c = c;
-  mk.s = F.stream;
-  const bool profiling = c->profiling;
-  c->profiling = false;  // stage events would serialise the streams
-  int rc = VBX_OK;
+  Marks mk{c, F.stream, false};  // no stage profiling: the events would serialise the streams
   // ---- front half on this scan's front lane
-  c->stream = F.stream;
-  c->apply_stream = nullptr;
-  c->sort_stream = nullptr;
   const float* dx = xyz;
   const uint8_t* dr = rgba;
   if (!on_device) {
@@ -2423,54 +2432,33 @@ int integrate_async(vbx_ctx* c, int kind, const float q[4], const float t[3], co
         cudaMemcpyAsync(S.d_rgba, rgba, (size_t)n * 4, cudaMemcpyHostToDevice, sc) != cudaSuccess ||
         cudaEventRecord(S.copy_done, sc) != cudaSuccess ||
         cudaStreamWaitEvent(F.stream, S.copy_done, 0) != cudaSuccess) {
-      rc = fail(c, VBX_E_CUDA, "asynchronous host-to-device copy failed");
+      return fail(c, VBX_E_CUDA, "asynchronous host-to-device copy failed");
     }
     dx = S.d_xyz;
     dr = S.d_rgba;
   }
   const uint64_t* keys64 = nullptr;
-  if (rc == VBX_OK && cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), F.stream) != cudaSuccess) {
-    rc = fail(c, VBX_E_CUDA, "cudaMemsetAsync");
-  }
-  if (rc == VBX_OK && c->timeline) cudaEventRecord(S.front_start, F.stream);
-  if (rc == VBX_OK) {
-    rc = front_half<uint64_t>(c, P, dx, dr, nullptr, mk, &launches, &keys64);
-  }
-  if (rc == VBX_OK && cudaEventRecord(S.front_done, F.stream) != cudaSuccess) rc = fail(c, VBX_E_CUDA, "cudaEventRecord");
+  if (cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), F.stream) != cudaSuccess) return fail(c, VBX_E_CUDA, "cudaMemsetAsync");
+  if (c->timeline) cudaEventRecord(S.front_start, F.stream);
+  if (int rc = front_half<uint64_t>(c, S, F, F.stream, P, dx, dr, nullptr, mk, &launches, &keys64)) return rc;
+  if (cudaEventRecord(S.front_done, F.stream) != cudaSuccess) return fail(c, VBX_E_CUDA, "cudaEventRecord");
   // ---- walk + record sort on stream_e, apply on the main stream
-  c->stream = c->stream_e;
-  c->sort_stream = c->stream_s[c->async_seq % vbx_ctx::kSortStreams];
-  c->walked_event = S.walked;
-  c->apply_stream = c->stream_main;
-  c->sorted_event = S.sorted;
-  mk.s = c->stream_e;
-  if (rc == VBX_OK && cudaStreamWaitEvent(c->stream_e, S.front_done, 0) != cudaSuccess) {
-    rc = fail(c, VBX_E_CUDA, "cudaStreamWaitEvent");
-  }
-  if (rc == VBX_OK) {
-    // Scans run their map-touching stages in submission order on this stream.  A scan that cannot be
-    // applied asynchronously (more update records than one pass holds) raises the context's hold
-    // flag here; every scan queued behind it then skips its back half, and the host redoes all of
-    // them synchronously, in order, from the retained inputs (recover_async, vbx_capi.cu).
-    if (rc == VBX_OK) {
-      k_back_begin<<<1, 1, 0, c->stream_e>>>(S.d_state, c->d_hold);
-      launches += 1;
-      rc = back_half<uint64_t>(c, P, keys64, 0, 0, mk, &launches);
-    }
-  }
+  if (cudaStreamWaitEvent(c->stream_e, S.front_done, 0) != cudaSuccess) return fail(c, VBX_E_CUDA, "cudaStreamWaitEvent");
+  // Scans run their map-touching stages in submission order on this stream.  A scan that cannot be
+  // applied asynchronously (more update records than one pass holds) raises the context's hold
+  // flag here; every scan queued behind it then skips its back half, and the host redoes all of
+  // them synchronously, in order, from the retained inputs (recover_async, vbx_capi.cu).
+  k_back_begin<<<1, 1, 0, c->stream_e>>>(S.d_state, c->d_hold);
+  launches += 1;
+  const Stages st{c->stream_e, c->stream_s[c->async_seq % vbx_ctx::kSortStreams], c->stream_main, S.walked, S.sorted};
+  if (int rc = back_half<uint64_t>(c, S, st, P, keys64, 0, 0, mk, &launches)) return rc;
   // the status block travels on a stream of its own: a copy between two scans' apply kernels would make the
   // apply stream (the pace setter of the pipeline) hop between the compute and the copy engine for every scan
-  if (rc == VBX_OK && (cudaEventRecord(S.applied, c->stream_main) != cudaSuccess ||
-                       cudaStreamWaitEvent(c->stream_h, S.applied, 0) != cudaSuccess ||
-                       cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, c->stream_h) != cudaSuccess ||
-                       cudaEventRecord(S.back_done, c->stream_h) != cudaSuccess)) {
-    rc = fail(c, VBX_E_CUDA, "enqueueing the result read-back failed");
+  if (cudaEventRecord(S.applied, c->stream_main) != cudaSuccess || cudaStreamWaitEvent(c->stream_h, S.applied, 0) != cudaSuccess ||
+      cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, c->stream_h) != cudaSuccess ||
+      cudaEventRecord(S.back_done, c->stream_h) != cudaSuccess) {
+    return fail(c, VBX_E_CUDA, "enqueueing the result read-back failed");
   }
-  c->profiling = profiling;
-  c->stream = c->stream_main;
-  c->apply_stream = nullptr;
-  c->sort_stream = nullptr;
-  if (rc != VBX_OK) return rc;
   S.in_flight = true;
   S.kind = kind;
   S.launches = launches;
@@ -2486,7 +2474,7 @@ int integrate_async(vbx_ctx* c, int kind, const float q[4], const float t[3], co
   c->launches += launches;
   c->async_seq += 1;
   if (c->deferred_rc) {
-    rc = c->deferred_rc;
+    const int rc = c->deferred_rc;
     c->err = c->deferred_msg;
     c->deferred_rc = 0;
     return rc;
@@ -2508,26 +2496,28 @@ __global__ void k_debug_order_setup(OrderScratch g, uint32_t n, ScanState* st) {
 }
 
 int debug_bundle_order(vbx_ctx* c, const uint32_t* hashes, uint32_t n, int force_global, uint32_t* out) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
+  vbx_ctx::ScratchSet& S = c->set[0];
+  const OrderScratch& g0 = c->lane[0].order_scratch;
   if (n > c->max_points) return fail(c, VBX_E_CAPACITY, "debug_bundle_order: n > max_points_per_scan");
   if (n == 0) return VBX_OK;
-  VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
-  VBX_CUDA(c, cudaMemcpyAsync(c->order_scratch.h, hashes, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-  k_debug_order_setup<<<grid_for(n, 256), 256, 0, s>>>(c->order_scratch, n, c->d_state);
+  VBX_CUDA(c, cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), s));
+  VBX_CUDA(c, cudaMemcpyAsync(g0.h, hashes, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+  k_debug_order_setup<<<grid_for(n, 256), 256, 0, s>>>(g0, n, S.d_state);
   RehashSchedule rs = c->rehash;
-  OrderScratch g = c->order_scratch;
+  OrderScratch g = g0;
   uint32_t smem_words = force_global ? 0u : (uint32_t)(c->order_smem_bytes / 4);
-  uint32_t* ray_list = c->ray_list;
-  uint32_t* cta_tot = c->order_scratch.cta_tot;
-  ScanState* st = c->d_state;
+  uint32_t* ray_list = S.ray_list;
+  uint32_t* cta_tot = g0.cta_tot;
+  ScanState* st = S.d_state;
   void* args[] = {&rs, &g, &smem_words, &ray_list, &cta_tot, &st};
   VBX_CUDA(c, cudaLaunchCooperativeKernel((void*)k_bundle_order, dim3(kOrderGrid), dim3(kOrderThreads), args,
                                           c->order_smem_bytes, s));
-  VBX_CUDA(c, cudaMemcpyAsync(out, c->ray_list, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-  VBX_CUDA(c, cudaMemcpyAsync(c->h_state, c->d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(out, S.ray_list, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(S.h_state, S.d_state, sizeof(ScanState), cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
   VBX_CUDA(c, cudaGetLastError());
-  if (c->h_state->error) return fail(c, VBX_E_CAPACITY, "debug_bundle_order: table capacity");
+  if (S.h_state->error) return fail(c, VBX_E_CAPACITY, "debug_bundle_order: table capacity");
   return VBX_OK;
 }
 
@@ -2540,31 +2530,33 @@ __global__ void k_iota(uint32_t* v, uint32_t n) {
 // record buffers with the count in device memory, 8 the point-key buffers with a host count.
 int debug_sort(vbx_ctx* c, const void* keys, int key_bytes, uint32_t n, int key_bits, void* keys_out,
                uint32_t* vals_out) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
+  vbx_ctx::ScratchSet& S = c->set[0];
+  vbx_ctx::FrontLane& F = c->lane[0];
   uint64_t launches = 0;
   if (key_bytes == 4) {
     if (n > c->max_updates) return fail(c, VBX_E_CAPACITY, "debug_sort: n > max_updates_per_pass");
-    VBX_CUDA(c, cudaMemcpyAsync(c->ckeys[0], keys, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-    k_iota<<<148, 256, 0, s>>>(c->cvals[0], n);
-    VBX_CUDA(c, cudaMemsetAsync(c->d_state, 0, sizeof(ScanState), s));
+    VBX_CUDA(c, cudaMemcpyAsync(S.ckeys[0], keys, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    k_iota<<<148, 256, 0, s>>>(S.cvals[0], n);
+    VBX_CUDA(c, cudaMemsetAsync(S.d_state, 0, sizeof(ScanState), s));
     const unsigned long long nn = n;
-    VBX_CUDA(c, cudaMemcpyAsync(&c->d_state->total_updates, &nn, sizeof(nn), cudaMemcpyHostToDevice, s));
-    if (int rc = own_sort<uint32_t>(c, 1, c->ckeys[0], c->cvals[0], c->ckeys[1], c->cvals[1],
-                                     &c->d_state->total_updates, 0, n, key_bits, true, &launches)) {
+    VBX_CUDA(c, cudaMemcpyAsync(&S.d_state->total_updates, &nn, sizeof(nn), cudaMemcpyHostToDevice, s));
+    if (int rc = own_sort<uint32_t>(c, s, S.sort_plan1, S.sort_status1, c->sort_tiles_cap[1], S.ckeys[0], S.cvals[0],
+                                     S.ckeys[1], S.cvals[1], &S.d_state->total_updates, 0, n, key_bits, true, &launches)) {
       return rc;
     }
-    VBX_CUDA(c, cudaMemcpyAsync(keys_out, c->ckeys[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-    VBX_CUDA(c, cudaMemcpyAsync(vals_out, c->cvals[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    VBX_CUDA(c, cudaMemcpyAsync(keys_out, S.ckeys[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    VBX_CUDA(c, cudaMemcpyAsync(vals_out, S.cvals[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
   } else if (key_bytes == 8) {
     if (n > c->max_points) return fail(c, VBX_E_CAPACITY, "debug_sort: n > max_points_per_scan");
-    VBX_CUDA(c, cudaMemcpyAsync(c->pkeys[0], keys, (size_t)n * 8, cudaMemcpyHostToDevice, s));
-    k_iota<<<148, 256, 0, s>>>(c->pvals[0], n);
-    if (int rc = own_sort<uint64_t>(c, 0, c->pkeys[0], c->pvals[0], c->pkeys[1], c->pvals[1], nullptr, n, n, key_bits, true,
-                                     &launches)) {
+    VBX_CUDA(c, cudaMemcpyAsync(S.pkeys0, keys, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+    k_iota<<<148, 256, 0, s>>>(F.pvals[0], n);
+    if (int rc = own_sort<uint64_t>(c, s, F.sort_plan0, F.sort_status0, c->sort_tiles_cap[0], S.pkeys0, F.pvals[0], F.pkeys1,
+                                     F.pvals[1], nullptr, n, n, key_bits, true, &launches)) {
       return rc;
     }
-    VBX_CUDA(c, cudaMemcpyAsync(keys_out, c->pkeys[0], (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-    VBX_CUDA(c, cudaMemcpyAsync(vals_out, c->pvals[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    VBX_CUDA(c, cudaMemcpyAsync(keys_out, S.pkeys0, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    VBX_CUDA(c, cudaMemcpyAsync(vals_out, F.pvals[0], (size_t)n * 4, cudaMemcpyDeviceToHost, s));
   } else {
     return fail(c, VBX_E_INVALID, "debug_sort: key_bytes must be 4 or 8");
   }
@@ -2575,17 +2567,19 @@ int debug_sort(vbx_ctx* c, const void* keys, int key_bytes, uint32_t n, int key_
 
 // exclusive prefix sum of n host uint32 through the engine's scan kernel
 int debug_scan(vbx_ctx* c, const uint32_t* in, uint32_t n, uint32_t* out) {
-  cudaStream_t s = c->stream;
+  cudaStream_t s = c->stream_main;
+  vbx_ctx::ScratchSet& S = c->set[0];
+  uint32_t* scan_status = c->lane[0].scan_status;
   if (n > c->max_points + 1) return fail(c, VBX_E_CAPACITY, "debug_scan: n > max_points_per_scan + 1");
-  VBX_CUDA(c, cudaMemcpyAsync(c->cnt, in, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+  VBX_CUDA(c, cudaMemcpyAsync(S.cnt, in, (size_t)n * 4, cudaMemcpyHostToDevice, s));
   const uint32_t tiles = (n + kScanTile - 1) / kScanTile;
-  VBX_CUDA(c, cudaMemsetAsync(c->scan_status, 0, (size_t)(tiles + 1) * sizeof(uint32_t), s));
+  VBX_CUDA(c, cudaMemsetAsync(scan_status, 0, (size_t)(tiles + 1) * sizeof(uint32_t), s));
   if (n) {
-    k_exclusive_scan<<<std::min<uint32_t>(tiles, 148 * 4), kSortThreads, 0, s>>>(c->cnt, nullptr, nullptr, c->off, n,
-                                                                               c->scan_status + 1, c->scan_status, nullptr,
+    k_exclusive_scan<<<std::min<uint32_t>(tiles, 148 * 4), kSortThreads, 0, s>>>(S.cnt, nullptr, nullptr, S.off, n,
+                                                                               scan_status + 1, scan_status, nullptr,
                                                                                nullptr, nullptr, 0ull, 0u);
   }
-  VBX_CUDA(c, cudaMemcpyAsync(out, c->off, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+  VBX_CUDA(c, cudaMemcpyAsync(out, S.off, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
   VBX_CUDA(c, cudaStreamSynchronize(s));
   VBX_CUDA(c, cudaGetLastError());
   return VBX_OK;
